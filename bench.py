@@ -18,9 +18,13 @@ With N > 1 GPUs the raster grows to (N*2048) x 2048 and is cut into N row bands,
          attenuation of the shortwave (specification ours: the reference has one AWS)
   configs.c5         BASELINE configs[4]: parameter ensemble on 4096 x 4096, 8 members per GPU; four members
          per pass of the fused kernel (enrgy_run_members)
-  --impl reference   the UNMODIFIED reference (baseline/_ref, copied by __graft_entry__.build()) run
+  --impl reference   the UNMODIFIED reference (oracle/_ref, copied by __graft_entry__.build()) run
          through oracle/ref_harness.py on the host cores -- per-step np.load of the insolation
-         and CSV appends included -- one process per core on row bands, on a bounded sample of C2.
+         and CSV appends included -- one process per core on row bands, on a bounded sample of C2;
+         without a copy of the reference, the NumPy oracle, reported as kind "port".
+  --dump-outputs DIR  the statistics and the glacier cells of the final state rasters of the headline's
+         last timed pass as .npy files (dump_outputs); the inputs are seeded, so two builds can be
+         compared output for output
 """
 from __future__ import annotations
 
@@ -274,6 +278,10 @@ def bench_c2(ctx, args, dtype, headline):
     cell_steps = float(n) * n * world * T
     value = cell_steps / (ms_step * 1e-3)
     stats_host = stats.cpu().numpy()
+    if headline and args.dump_outputs and ctx.rank == 0:
+        # before the e2e leg below, which uploads and runs the season again
+        dump_outputs(args.dump_outputs, stats_host, eng.state(np.float32 if precision == _lib.F32 else np.float64),
+                     ~np.isnan(case.dem))
     n_valid = float(np.count_nonzero(~np.isnan(case.dem)))
     bytes_per_launch = algorithmic_bytes(case, precision)
     peak = eng.microbench(0 if dtype == "f32" else 1) if ctx.rank == 0 else None
@@ -533,6 +541,32 @@ def run_ours(args):
         emit(result)
 
 
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_SEED = 0
+
+
+def dump_outputs(path, stats, state, valid):
+    """--dump-outputs: what the last timed pass hands its caller, as <path>/<name>.npy -- the per-step
+    area statistics (float64 [T, S_COUNT], all-reduced over ranks) and rank 0's final swe, total_snow and
+    total_ice rasters in the run's precision, at the glacier cells `valid` only (ascending cell index):
+    off the glacier the rasters are NaN by definition (model.py:258), and the DEM alone decides where.
+    Cells that would take the files over DUMP_BYTES are cut to the same seeded sample in every raster,
+    so two builds can be compared file by file."""
+    os.makedirs(path, exist_ok=True)
+    state = [a[valid] for a in state]
+    cells = state[0].size
+    room = (DUMP_BYTES - stats.nbytes - 4096) // (len(state) * state[0].itemsize)     # (4096: .npy headers)
+    if room < 1:
+        raise ValueError("--dump-outputs: the statistics alone (%d bytes) fill the %d-byte budget" % (stats.nbytes, DUMP_BYTES))
+    idx = None
+    if cells > room:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(cells, room, replace=False))
+    np.save(os.path.join(path, "stats.npy"), stats)
+    for name, a in zip(("swe", "total_snow", "total_ice"), state):
+        np.save(os.path.join(path, name + ".npy"), a if idx is None else a[idx])
+    log("outputs of the last timed pass written to %s%s" % (path, "" if idx is None else " (%d of %d cells)" % (room, cells)))
+
+
 def issue_roofline(cell_steps, kernel_ms, clocks, dtype):
     """The binding resources of the fused kernel (ncu: DRAM < 1 %): FP32-pipe lane-operations per
     second against 128 lanes x SMs x clock, and instruction issue slots against 4 schedulers x 32
@@ -571,7 +605,7 @@ def algorithmic_bytes(case, precision):
 
 
 # ---------------------------------------------------------------------------------------------
-# CPU arm: the unmodified reference (baseline/_ref) through oracle/ref_harness.py, or -- if that copy
+# CPU arm: the unmodified reference (oracle/_ref) through oracle/ref_harness.py, or -- if that copy
 # is absent -- the NumPy oracle (a restatement pinned bit-identically against the reference).
 _SAMPLE = {}
 
@@ -669,16 +703,13 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     n, T = args.n, args.t
     vals, secs = [], []
-    t_all = time.perf_counter()
     last = None
     cpu_sample(n, args.cpu_sample_steps)                 # (untimed: building the sample)
     for _ in range(args.warmup + args.steps):
         last = cpu_baseline(n, args.cpu_sample_steps, cores)
         vals.append(last["value"])
         secs.append(last["model_seconds"])
-        if time.perf_counter() - t_all > 200:
-            break
-    n_warm = min(args.warmup, max(len(vals) - 1, 0))
+    n_warm = args.warmup
     timed, tsecs = vals[n_warm:], secs[n_warm:]
     value = float(np.mean(timed))
     one = cpu_baseline(n, args.cpu_sample_steps, 1) if args.single_core else None
@@ -720,7 +751,13 @@ def main():
     ap.add_argument("--c4-t", type=int, default=2200)
     ap.add_argument("--c5-n", type=int, default=4096)
     ap.add_argument("--c5-members", type=int, default=8, help="ensemble members per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the statistics and state rasters of the last timed pass as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         log("note: the timing rules ask for >= 3 warm-up passes")
     if args.impl == "reference":

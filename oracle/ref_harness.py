@@ -31,10 +31,9 @@ _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _find_reference():
-    """The reference checkout (build container), else the unmodified copy __graft_entry__.build() puts
-    under baseline/_ref/ (git-ignored; it travels to the GPU box, where bench.py --impl reference and
-    the cpu_baseline leg time it)."""
-    for d in (os.environ.get("ENRGY_REFERENCE_DIR"), "/root/reference", os.path.join(_ROOT, "baseline", "_ref")):
+    """ENRGY_REFERENCE_DIR, else the declared reference checkout (BASELINE.json reference_path), else
+    the unmodified copy __graft_entry__.build() puts under oracle/_ref/ (git-ignored)."""
+    for d in (os.environ.get("ENRGY_REFERENCE_DIR"), "/root/reference", os.path.join(_ROOT, "oracle", "_ref")):
         if d and os.path.isfile(os.path.join(d, "model.py")):
             return d
     return os.environ.get("ENRGY_REFERENCE_DIR", "/root/reference")

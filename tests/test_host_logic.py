@@ -277,6 +277,46 @@ def test_ensemble_members_and_sharding():
     assert shard(a[:5], 8, 7) == [] and shard(a[:5], 2, 1) == [1, 3]
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: the glacier cells of the rasters (off it they are NaN by definition), all of
+    them while they fit the byte budget, else the same seeded sample of cells from every raster, the same
+    on every call; finite float32/float64 values only."""
+    import bench
+    rng = np.random.default_rng(5)
+    stats = rng.random((30, _lib.S_COUNT))
+    cells = 64 * 80
+    valid = (np.arange(cells) % 7 != 3).reshape(64, 80)
+    for dtype in (np.float32, np.float64):
+        # every value is its raster's number times `cells` plus its cell index; NaN off the glacier
+        state = tuple(np.where(valid, (np.arange(cells) + q * cells).reshape(64, 80), np.nan).astype(dtype)
+                      for q in range(3))
+        bench.dump_outputs(str(tmp_path / "whole"), stats, state, valid)
+        for name, a in zip(("swe", "total_snow", "total_ice"), state):
+            assert np.array_equal(np.load(tmp_path / "whole" / (name + ".npy")), a[valid])
+        assert np.array_equal(np.load(tmp_path / "whole" / "stats.npy"), stats)
+        monkeypatch.setattr(bench, "DUMP_BYTES", 40000)
+        runs = []
+        for k in range(2):
+            d = tmp_path / ("sample%d" % k)
+            bench.dump_outputs(str(d), stats, state, valid)
+            files = {f.name: np.load(f) for f in d.iterdir()}
+            assert sum(f.stat().st_size for f in d.iterdir()) <= 40000
+            assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in files.values())
+            runs.append(files)
+        monkeypatch.undo()
+        assert runs[0].keys() == runs[1].keys() == {"stats.npy", "swe.npy", "total_snow.npy", "total_ice.npy"}
+        assert all(np.array_equal(runs[0][k], runs[1][k]) for k in runs[0])
+        swe = runs[0]["swe.npy"]
+        assert swe.dtype == dtype and 0 < swe.size < valid.sum() and np.all(np.diff(swe) > 0)
+        assert valid.ravel()[swe.astype(int)].all()                             # glacier cells only
+        assert np.array_equal(runs[0]["total_snow.npy"], swe + cells)          # the same cells in each raster
+        assert np.array_equal(runs[0]["total_ice.npy"], swe + 2 * cells)
+        monkeypatch.setattr(bench, "DUMP_BYTES", stats.nbytes)                  # no room left for any cell
+        with pytest.raises(ValueError):
+            bench.dump_outputs(str(tmp_path / "full"), stats, state, valid)
+        monkeypatch.undo()
+
+
 def test_header_is_plain_c(tmp_path):
     """include/enrgy_b200.h is the drop-in boundary: it must compile as C11 and as C++17 on its own, and the
     calls INTEGRATION.md shows must match its prototypes."""
