@@ -360,7 +360,6 @@ int fill_args(enrgy_ctx* c, int t0, int t1, KernelArgs<R>& a) {
   a.msm.inv_snow_density = (R)(1.0 / c->p.snow_density);
   a.msm.g0_ice = a.msm.k_ice * a.msm.c_ice * a.msm.rho_ice;
   a.msm.crd_ice = a.msm.c_ice * a.msm.rho_ice * a.msm.d[0];
-  a.msm.inv_crd_ice = (R)1 / a.msm.crd_ice;
   a.steps = (const StepRec<R>*)c->d_steps.p;
   a.subs = (const SubRec<R>*)c->d_subs.p;
   a.blocks = c->d_blocks.p;
@@ -473,7 +472,12 @@ int sweep_range(enrgy_ctx* c, int sub0, int sub1, int n_seg, const SweepSeg* seg
   auto by_direction = [](const SweepSub& x, const SweepSub& y) { return x.sigma != y.sigma ? x.sigma < y.sigma : x.dfix < y.dfix; };
   std::stable_sort(row_subs.begin(), row_subs.end(), by_direction);
   std::stable_sort(col_subs.begin(), col_subs.end(), by_direction);
-  for (size_t i = 0; i < col_subs.size(); ++i) col_subs[i].out = (int)i;   // slot in the transposed temporary
+  // the sub-steps go to launch_sweep in slices of at most kSweepMaxRowSubs / kSweepMaxColSubs (CUDA grid
+  // limits; a long run on a small raster holds millions of sub-steps in one chunk); the column-type ones
+  // of a slice share one transposed temporary
+  for (size_t i = 0; i < col_subs.size(); ++i) col_subs[i].out = (int)(i % kSweepMaxColSubs);   // slot in it
+  const size_t n_slices = std::max((row_subs.size() + kSweepMaxRowSubs - 1) / kSweepMaxRowSubs,
+                                   (col_subs.size() + kSweepMaxColSubs - 1) / kSweepMaxColSubs);
   SweepArgs a{};
   a.rows = c->rows; a.cols = c->cols;
   a.scan = c->d_scan.p + (size_t)kScanRowApron * scan_pitch(c->cols) + kScanColApron;
@@ -485,10 +489,8 @@ int sweep_range(enrgy_ctx* c, int sub0, int sub1, int n_seg, const SweepSeg* seg
   // (pageable source: the copy is staged before the call returns, the vectors may go out of scope)
   if (!row_subs.empty()) CU_TRY(cudaMemcpyAsync(c->d_sweepsubs.p, row_subs.data(), row_subs.size() * sizeof(SweepSub), cudaMemcpyHostToDevice, stream));
   if (!col_subs.empty()) CU_TRY(cudaMemcpyAsync(c->d_sweepsubs.p + row_subs.size(), col_subs.data(), col_subs.size() * sizeof(SweepSub), cudaMemcpyHostToDevice, stream));
-  a.row_subs = c->d_sweepsubs.p; a.n_row_subs = (int)row_subs.size();
-  a.col_subs = c->d_sweepsubs.p + row_subs.size(); a.n_col_subs = (int)col_subs.size();
   if (!col_subs.empty()) {
-    CU_TRY(c->d_masktmp.alloc(col_subs.size() * (size_t)c->cols * a.tmp_words));
+    CU_TRY(c->d_masktmp.alloc(std::min(col_subs.size(), (size_t)kSweepMaxColSubs) * (size_t)c->cols * a.tmp_words));
     a.tmp = c->d_masktmp.p;
   }
   for (int z : zenith) {
@@ -497,12 +499,19 @@ int sweep_range(enrgy_ctx* c, int sub0, int sub1, int n_seg, const SweepSeg* seg
       CU_TRY(cudaMemsetAsync(segs[q].ptr + (size_t)z * words, 0xFF, words * sizeof(unsigned), stream));
     }
   }
-  int n = 0;
   CU_TRY(sweep_events(c).begin(stream));
-  CU_TRY(launch_sweep(a, c->sm_count, stream, &n));
+  for (size_t k = 0; k < n_slices; ++k) {
+    // (stream order: the transpose of slice k has read the temporary before slice k + 1 sweeps into it)
+    const size_t r0 = std::min(row_subs.size(), k * kSweepMaxRowSubs), r1 = std::min(row_subs.size(), r0 + kSweepMaxRowSubs);
+    const size_t c0 = std::min(col_subs.size(), k * kSweepMaxColSubs), c1 = std::min(col_subs.size(), c0 + kSweepMaxColSubs);
+    a.row_subs = c->d_sweepsubs.p + r0; a.n_row_subs = (int)(r1 - r0);
+    a.col_subs = c->d_sweepsubs.p + row_subs.size() + c0; a.n_col_subs = (int)(c1 - c0);
+    int n = 0;
+    CU_TRY(launch_sweep(a, c->sm_count, stream, &n));
+    c->launches += n;
+    c->sweep_launches += n;
+  }
   CU_TRY(sweep_events(c).end(stream));
-  c->launches += n;
-  c->sweep_launches += n;
   return ENRGY_OK;
 }
 
@@ -952,6 +961,8 @@ int enrgy_set_params(enrgy_ctx* c, const enrgy_params* pin) {
   if (p.insol_mode != ENRGY_INSOL_STREAMED && p.insol_mode != ENRGY_INSOL_COMPUTED) return fail(ENRGY_ERR_ARG, "bad insol_mode");
   if (p.band_rows == 0) { p.band_row0 = 0; p.band_rows = c->rows; }
   if (p.band_row0 < 0 || p.band_rows < 0 || p.band_row0 + p.band_rows > c->rows) return fail(ENRGY_ERR_ARG, "row band outside the raster");
+  // the sweep writes the sunlit masks in groups of 8 raster rows (shade.cu)
+  if (p.shadow && (p.band_row0 & 7)) return fail(ENRGY_ERR_ARG, "with shading the row band must start on a multiple of 8 rows (band_row0 = %d)", p.band_row0);
   c->p = p;
   c->albedo_offset = 0.0;
   c->base_albedo_ice = p.albedo_ice; c->base_albedo_snow = p.albedo_snow;

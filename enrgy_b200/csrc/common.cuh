@@ -61,7 +61,7 @@ struct MsmParams {
   R inv_snow_density;                         // snow depth = swe / snow_density (model.py:428, sic)
   // surface layer of a snow-free cell (snow share 0: conductivity and density are those of ice exactly)
   R g0_ice;                                   // k_ice * c_ice * rho_ice: in-glacier flux per unit temperature gradient
-  R crd_ice, inv_crd_ice;                     // c_ice * rho_ice * d[0] (heat capacity of the layer per m2) and 1 / it
+  R crd_ice;                                  // c_ice * rho_ice * d[0] (heat capacity of the layer per m2)
 };
 
 // ---- per-step record (24 values, staged per time block by a TMA bulk copy) ---------------------

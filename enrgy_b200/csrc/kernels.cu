@@ -1120,7 +1120,10 @@ energy_balance_kernel(const KernelArgs<R> a) {
             // Snow-free cells (the ablation zone for most of the season): the snow share of every layer is 0,
             // conductivity and density are those of ice exactly, and the surface layer of the pair runs
             // packed with per-run constants -- 8 packed operations instead of ~70 scalar ones.  Decided per
-            // warp, so a cell's arithmetic depends on its patch only (bit-identical across bands and cuts).
+            // warp, and which cells share a warp depends on where a row band starts and ends: so this path
+            // performs, operation for operation, the general path's arithmetic at a snow share of 0 (its
+            // constants are that path's intermediates exactly, the reciprocal the same approximation),
+            // and a cell's result does not depend on the decision.
             const bool bare = !__any_sync(0xffffffffu, snow_lo || snow_hi);
             if (bare) {
               const V t0v = V::make(tl[2 * q][0], tl[2 * q + 1][0]), t1v = V::make(tl[2 * q][1], tl[2 * q + 1][1]);
@@ -1130,7 +1133,7 @@ energy_balance_kernel(const KernelArgs<R> a) {
               // melt gate: qm = full - q0, q0 = -t0 c rho d / dt (msm.py:88-93)
               const V gate = fma2(t0v, V::splat(mp.crd_ice * inv_dt), full);
               const V mfv = V::make(fmax_(gate.lo(), (R)0), fmax_(gate.hi(), (R)0));
-              const V dlt = mul2(sub2(full, mfv), V::splat(mp.inv_crd_ice));
+              const V dlt = mul2(sub2(full, mfv), V::splat(Num<R>::rcp(mp.crd_ice)));
 #pragma unroll
               for (int h = 0; h < 2; ++h) {
                 const int i = 2 * q + h;
@@ -1160,10 +1163,11 @@ energy_balance_kernel(const KernelArgs<R> a) {
               const V below = sub2(sd, d0_2);
               const V grad = mul2(sub2(t1v, t0v), inv_d0);                                              // msm.py:18-28
               const V c_ice2 = V::splat(mp.c_ice);
-              const V gv = mul2(mul2(mul2(kap, grad), c_ice2), rho);
+              // (association as in the snow-free path above: kap c rho is g0_ice, c rho d is crd_ice at no snow)
+              const V gv = mul2(grad, mul2(mul2(kap, c_ice2), rho));
               const V full = add2(atmo, gv);
               const V crd = mul2(mul2(c_ice2, rho), d0_2);
-              const V gate = fma2(mul2(t0v, crd), V::splat(inv_dt), full);          // full - q0, q0 = -t0 c rho d / dt
+              const V gate = fma2(t0v, mul2(crd, V::splat(inv_dt)), full);          // full - q0, q0 = -t0 c rho d / dt
               const V mfv = V::make(fmax_(gate.lo(), (R)0), fmax_(gate.hi(), (R)0));
               const V dlt = mul2(sub2(full, mfv), V::make(Num<R>::rcp(crd.lo()), Num<R>::rcp(crd.hi())));
 #pragma unroll
@@ -1220,7 +1224,7 @@ energy_balance_kernel(const KernelArgs<R> a) {
                     sd = fmax_(sd - mp.d[l], (R)0);
                     const R dlt = kap * (grad - grad_prev) * mp.inv_d[l];
                     grad_prev = grad;
-                    tl[i][l] = t_here + dlt * dt;
+                    tl[i][l] = fma(dlt, dt, t_here);              // (as the packed loop above)
                   }
                 }
               }

@@ -199,6 +199,10 @@ struct SweepArgs {
   int tmp_words;             // round_up(ceil(rows / 32), 8)
 };
 inline int sweep_tmp_words(int rows) { return ((rows + 31) / 32 + 7) / 8 * 8; }
+// sub-steps one launch_sweep takes: the transpose runs one grid.z slice per column-type sub-step and the
+// sweep one grid.y row per 4 row-type sub-steps, and CUDA caps both grid dimensions at 65535
+constexpr int kSweepMaxColSubs = 65535;
+constexpr int kSweepMaxRowSubs = 4 * 65535;
 cudaError_t launch_sweep(const SweepArgs& a, int sm_count, cudaStream_t stream, int* n_launches);
 cudaError_t launch_microbench(int kind, int sm_count, int iters, void* scratch, double* ops_per_launch,
                               cudaStream_t stream);

@@ -324,6 +324,7 @@ cudaError_t launch_sweep(const SweepArgs& a, int sm_count, cudaStream_t stream, 
   (void)sm_count;
   constexpr int V = ENRGY_SWEEP_V, U = ENRGY_SWEEP_U, Q = ENRGY_SWEEP_Q;
   static_assert(U <= kScanRowApron && 32 * V + 32 <= kScanColApron, "aprons of the scan copy");
+  static_assert((long long)Q * 65535 >= kSweepMaxRowSubs, "grid.y of the sweep");
   int n = 0;
   // line groups: windows of 32 V lines every 32 (V - 1) lines over [-sh_max, nb - sh_min); the shear
   // spans at most the length of the sweep axis (|dfix| <= 65536)

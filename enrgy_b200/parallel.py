@@ -42,8 +42,9 @@ def row_bands(rows, world, align=16, valid_per_row=None):
         target = total * r / world
         e = int(np.searchsorted(cum, target))
         e = int(round(e / align)) * align
-        # every band keeps at least `align` rows, also where the glacier occupies a few rows only
-        e = min(max(e, edges[-1] + align), rows - (world - r) * align)
+        # every band keeps at least `align` rows, also where the glacier occupies a few rows only; the
+        # upper bound is rounded down to a multiple of `align` too (rows need not be one)
+        e = min(max(e, edges[-1] + align), (rows // align - (world - r)) * align)
         edges.append(e)
     edges.append(rows)
     return [(edges[i], edges[i + 1] - edges[i]) for i in range(world)]

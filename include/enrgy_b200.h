@@ -142,7 +142,8 @@ typedef struct enrgy_params {
   int32_t _pad2;
   double msm_depths[ENRGY_MAX_LAYERS];
   /* --- row band of a larger raster (multi-GPU, SURVEY 8e) --- */
-  int32_t band_row0;     /* first row of this handle's band inside the full DEM */
+  int32_t band_row0;     /* first row of this handle's band inside the full DEM; a multiple of 8
+                            when shadow != 0 (enrgy_set_params returns ENRGY_ERR_ARG otherwise) */
   int32_t band_rows;     /* rows of the band; 0 = whole raster */
 } enrgy_params;
 

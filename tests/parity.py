@@ -93,6 +93,10 @@ def make_engine(case, f64, pot=None, computed=False, shadow=False, device=0, ban
         eng.set_insolation(0, np.ascontiguousarray(np.asarray(pot, dtype=np.float32)[:, rows]))
         if band is not None:
             eng.set_insolation_aws(0, np.asarray(pot, dtype=np.float32)[:, case.aws_rc[0], case.aws_rc[1]])
+    if kw.get("msm") and band is not None:
+        # the sub-surface pre-pass integrates the AWS cell on every band (as Energy.model hands it over)
+        ar, ac = case.aws_rc
+        eng.set_aws_cell([float(alb[k][ar, ac]) for k in keys] if keys else None, float(case.swe[ar, ac]))
     eng.prepass()
     return eng
 
@@ -141,17 +145,46 @@ def random_insolation(case, n_steps, seed=5, f32=True):
     return pot
 
 
-def compare_run(case, f64, pot=None, computed=False, shadow=False, **kw):
-    """Runs oracle and engine; returns dict of worst relative errors."""
+def oracle_insolation(case, pot, computed, shadow, f64):
+    """The insolation the oracle runs on: `pot` when it is streamed, else the specification's series."""
+    if not computed:
+        return pot
+    pot_o = I.insolation_series(case, shadow=shadow, dtype=np.float64)
+    return pot_o if f64 else pot_o.astype(np.float32)
+
+
+def oracle_band_sums(ora, rows, valid):
+    """[T, S_COUNT] statistics of the rows `rows` of the raster, as float64 sums of the oracle's per-step
+    rasters (flux sums over glacier cells, SWE sums and counts over its non-NaN cells, before the update)."""
+    v = valid[rows]
+    out = np.zeros((len(ora["rows"]), _lib.S_COUNT))
+    cols = ((_lib.S_RS, "rs"), (_lib.S_LWD, "lwd"), (_lib.S_LWU, "lwu"), (_lib.S_SENS, "sens"),
+            (_lib.S_LAT, "lat"), (_lib.S_ATMO, "atmo"), (_lib.S_G, "g"), (_lib.S_MELT, "mf"))
+    for i, (r, (snow, ice, swe)) in enumerate(zip(ora["rows"], ora["melt"])):
+        for col, name in cols:
+            out[i, col] = np.nansum(np.asarray(r[name], dtype=np.float64)[rows][v])
+        out[i, _lib.S_SNOW] = np.nansum(np.asarray(snow, dtype=np.float64)[rows][v])
+        out[i, _lib.S_ICE] = np.nansum(np.asarray(ice, dtype=np.float64)[rows][v])
+        swe = np.asarray(swe, dtype=np.float64)[rows]
+        out[i, _lib.S_SWE] = np.nansum(swe)
+        out[i, _lib.S_NSNOW] = np.count_nonzero(swe > 0)
+        out[i, _lib.S_NSWE] = np.count_nonzero(~np.isnan(swe))
+        out[i, _lib.S_NVALID] = np.count_nonzero(v)
+    return out
+
+
+def compare_run(case, f64, pot=None, computed=False, shadow=False, band=None, ora=None, **kw):
+    """Runs oracle and engine; returns dict of worst relative errors.
+    band = (row0, rows): the engine runs that row band; its rasters are compared with those rows of the
+    whole-raster oracle and its statistics with the oracle's float64 sums over them ("band_sums"; the
+    glacier-wide means only exist for the whole raster).  ora: run_oracle's result for these inputs, for
+    callers that compare several bands against one oracle run."""
     n = len(case.aws_rows)
-    if computed:
-        pot_o = I.insolation_series(case, shadow=shadow, dtype=np.float64)
-        if not f64:
-            pot_o = pot_o.astype(np.float32)
-    else:
-        pot_o = pot
-    ora = run_oracle(case, pot_o, f64, **kw)
-    eng = make_engine(case, f64, pot=pot, computed=computed, shadow=shadow, **kw)
+    r0, nr = band if band is not None else (0, case.shape[0])
+    rows = slice(r0, r0 + nr)
+    if ora is None:
+        ora = run_oracle(case, oracle_insolation(case, pot, computed, shadow, f64), f64, **kw)
+    eng = make_engine(case, f64, pot=pot, computed=computed, shadow=shadow, band=band, **kw)
     try:
         dump = eng.dump_steps(0, n)
         stats = eng.run(0, n)
@@ -167,19 +200,18 @@ def compare_run(case, f64, pot=None, computed=False, shadow=False, **kw):
         # very case (SURVEY 8c): the as-shipped reference deviates from its float64-injected self by a few
         # 1e-3 W m-2 in the melt flux (the gate carries the cold content of the surface layer, which integrates
         # the float32 round-off of every earlier step).  1e-4 x 5 W m-2 = 5e-4 W m-2 must not be looser than that.
-        ora64 = run_oracle(case, pot_o if not computed else I.insolation_series(case, shadow=shadow, dtype=np.float64),
-                           True, **kw)
+        ora64 = run_oracle(case, oracle_insolation(case, pot, computed, shadow, True), True, **kw)
         own_gap = max(float(np.nanmax(np.abs(np.asarray(a["mf"], dtype=np.float64) - b["mf"])))
                       for a, b in zip(ora["rows"], ora64["rows"]))
         assert 1e-4 * msm_floor <= own_gap, ("the float32 melt-flux bound is looser than the reference's own float32 "
                                              "error on this case", own_gap)
     res = {}
-    off = np.isnan(case.dem)
+    off = np.isnan(case.dem)[rows]
     for name in FLUX_FIELDS:
         idx = _lib.DUMP_NAMES.index(name)
         worst = 0.0
         for i in range(n):
-            ref = np.array(ora["rows"][i][name], dtype=np.float64)
+            ref = np.array(ora["rows"][i][name], dtype=np.float64)[rows]
             if name == "g" and not kw.get("msm"):
                 ref[off] = np.nan       # np.zeros(atmo.shape): finite off-glacier (model.py:434)
             if name == "lwu" and not kw.get("msm"):
@@ -198,24 +230,36 @@ def compare_run(case, f64, pot=None, computed=False, shadow=False, **kw):
         res[name] = worst
     worst = 0.0
     for i in range(n):
-        ref = np.array(ora["rows"][i]["albedo"], dtype=np.float64)
+        ref = np.array(ora["rows"][i]["albedo"], dtype=np.float64)[rows]
         ref[off] = np.nan           # constant-albedo rasters are finite off-glacier (model.py:332)
         worst = max(worst, max_rel_err(dump[i, _lib.D_ALBEDO], ref, 1e-3))
     res["albedo"] = worst
-    res["snow"] = max(max_rel_err(dump[i, _lib.D_SNOW], ora["melt"][i][0], mfl) for i in range(n))
-    res["ice"] = max(max_rel_err(dump[i, _lib.D_ICE], ora["melt"][i][1], mfl) for i in range(n))
+    res["snow"] = max(max_rel_err(dump[i, _lib.D_SNOW], ora["melt"][i][0][rows], mfl) for i in range(n))
+    res["ice"] = max(max_rel_err(dump[i, _lib.D_ICE], ora["melt"][i][1][rows], mfl) for i in range(n))
     if layers is not None:
-        res["layer_t"] = max(max_rel_err(layers[l], ora["layer_temperatures"][l], 1e-3 if f64 else 1.0)
+        res["layer_t"] = max(max_rel_err(layers[l], ora["layer_temperatures"][l][rows], 1e-3 if f64 else 1.0)
                              for l in range(layers.shape[0]))
-    res["swe"] = max_rel_err(swe, ora["swe"], tfl)
-    res["total_snow"] = max_rel_err(tsn, ora["total_snow"], tfl)
-    res["total_ice"] = max_rel_err(tic, ora["total_ice"], tfl)
-    res["total_ice_l2"] = l2_rel_err(tic, ora["total_ice"])
-    res["total_snow_l2"] = l2_rel_err(tsn, ora["total_snow"])
-    m_e = means_from_stats(stats)
-    m_o = ora["means"]
-    floors = np.array([ff, ff, ff, ff, ff, ff, ff, ff, mfl, mfl, tfl, 0.5, 0.5])
-    res["means"] = float(np.max(np.abs(m_e - m_o) / np.maximum(np.abs(m_o), floors)))
+    res["swe"] = max_rel_err(swe, ora["swe"][rows], tfl)
+    res["total_snow"] = max_rel_err(tsn, ora["total_snow"][rows], tfl)
+    res["total_ice"] = max_rel_err(tic, ora["total_ice"][rows], tfl)
+    res["total_ice_l2"] = l2_rel_err(tic, ora["total_ice"][rows])
+    res["total_snow_l2"] = l2_rel_err(tsn, ora["total_snow"][rows])
+    if band is None:
+        m_e = means_from_stats(stats)
+        m_o = ora["means"]
+        floors = np.array([ff, ff, ff, ff, ff, ff, ff, ff, mfl, mfl, tfl, 0.5, 0.5])
+        res["means"] = float(np.max(np.abs(m_e - m_o) / np.maximum(np.abs(m_o), floors)))
+    else:
+        s_o = oracle_band_sums(ora, rows, ~np.isnan(case.dem))
+        # the per-cell floors, times the cells a sum runs over
+        floors = np.full(_lib.S_COUNT, ff)
+        if kw.get("msm") and not f64:
+            floors[[_lib.S_MELT, _lib.S_G]] = msm_floor
+        floors[[_lib.S_SNOW, _lib.S_ICE]] = mfl
+        floors[_lib.S_SWE] = tfl
+        floors[[_lib.S_NSNOW, _lib.S_NSWE, _lib.S_NVALID]] = 0.5
+        scale = np.maximum(s_o[:, [_lib.S_NVALID]], 1.0)
+        res["band_sums"] = float(np.max(np.abs(stats - s_o) / np.maximum(np.abs(s_o), floors * scale)))
     res["L"] = float(np.max(np.abs(point[:, _lib.P_L] - [r["L"] for r in ora["rows"]])
                             / np.abs([r["L"] for r in ora["rows"]])))
     return res

@@ -160,16 +160,22 @@ def test_tile_cost_weights():
 def test_band_cuts_properties_randomised():
     """row_bands / rebalance_bands on random weights and times: bands tile the raster without gaps or
     overlaps, edges are aligned, no band is empty, and re-cutting with the times a perfectly
-    uniform cost model would have produced leaves the bands unchanged."""
-    from hypothesis import given, settings, strategies as st
+    uniform cost model would have produced leaves the bands unchanged.  Raster heights need not be a
+    multiple of the alignment (the weight in the bottom rows pulls the cuts against the upper bound)."""
+    from hypothesis import example, given, settings, strategies as st
 
     @settings(max_examples=60, deadline=None)
-    @given(st.integers(1, 8), st.integers(1, 40), st.integers(0, 2**31 - 1), st.sampled_from([1, 8, 16]))
-    def check(world, groups, seed, align):
-        rows = groups * 16
+    @given(st.integers(1, 8), st.integers(1, 40), st.integers(0, 15), st.integers(0, 2**31 - 1),
+           st.sampled_from([1, 8, 16]), st.booleans())
+    @example(2, 6, 4, 0, 16, True)                   # rows = 100: once cut at row 84
+    @example(3, 16, 1, 0, 16, True)                  # rows = 257: once cut at rows 225 and 241
+    def check(world, groups, extra, seed, align, bottom):
+        rows = groups * 16 + extra
         rng = np.random.default_rng(seed)
         w = rng.integers(0, 200, rows).astype(float)
         w[rng.random(rows) < 0.3] = 0.0
+        if bottom:
+            w[:rows - min(rows, 16)] = 0.0           # all the weight in the last rows
         if rows < world * align:
             with pytest.raises(ValueError):
                 row_bands(rows, world, align=align, valid_per_row=w)
