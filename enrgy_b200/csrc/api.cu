@@ -48,6 +48,10 @@ template <typename T>
 struct DevBuf {
   T* p = nullptr;
   size_t n = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { release(); }
   cudaError_t alloc(size_t count) {
     if (count <= n && p) return cudaSuccess;
     release();
@@ -59,6 +63,48 @@ struct DevBuf {
     if (p) cudaFree(p);
     p = nullptr;
     n = 0;
+  }
+};
+
+// ---- CUDA event pairs around the kernels of the last run (several chunks -> several pairs) ---------
+struct EventPairs {
+  std::vector<cudaEvent_t> ev;   // begin, end, begin, end, ...
+  int used = 0;
+  bool pending = false;
+  double last_ms = 0.0;
+  void reset() { used = 0; pending = false; }
+  cudaError_t begin(cudaStream_t s) {
+    while ((int)ev.size() < used + 2) {
+      cudaEvent_t e;
+      cudaError_t rc = cudaEventCreate(&e);
+      if (rc != cudaSuccess) return rc;
+      ev.push_back(e);
+    }
+    return cudaEventRecord(ev[used], s);
+  }
+  cudaError_t end(cudaStream_t s) {
+    cudaError_t rc = cudaEventRecord(ev[used + 1], s);
+    used += 2;
+    pending = true;
+    return rc;
+  }
+  double collect() {
+    if (pending) {
+      double tot = 0.0;
+      for (int i = 0; i + 1 < used; i += 2) {
+        float ms = 0.f;
+        if (cudaEventSynchronize(ev[i + 1]) == cudaSuccess && cudaEventElapsedTime(&ms, ev[i], ev[i + 1]) == cudaSuccess) tot += ms;
+      }
+      last_ms = tot;
+      pending = false;
+    }
+    return last_ms;
+  }
+  EventPairs() = default;
+  EventPairs(const EventPairs&) = delete;
+  EventPairs& operator=(const EventPairs&) = delete;
+  ~EventPairs() {
+    for (cudaEvent_t e : ev) cudaEventDestroy(e);
   }
 };
 
@@ -101,7 +147,6 @@ struct enrgy_ctx {
   // a run cut into several launches: SWE at its start (total_snow = start - end is added by the last)
   DevBuf<unsigned char> d_swe_ref;
   int defer = 0;                  // 0 off, 1 deferring (launches leave total_snow alone), 2 the next launch applies
-  int64_t sweep_launches = 0;
   DevBuf<unsigned char> d_nx, d_ny, d_nz, d_swe, d_ts, d_ti, d_dump, d_stage, d_snap, d_layer_t;
   bool have_msm = false;
   std::vector<double> alb_aws, layer_t_aws;
@@ -112,7 +157,6 @@ struct enrgy_ctx {
   // tables
   DevBuf<unsigned char> d_steps, d_subs;
   DevBuf<StepRec<double>> d_steps64;
-  DevBuf<ShadeRec> d_shades;
   DevBuf<TimeBlock> d_blocks;
   DevBuf<int2> d_tiles;
   DevBuf<int> d_counts;
@@ -137,23 +181,55 @@ struct enrgy_ctx {
   DevBuf<unsigned char> d_partials;
   DevBuf<unsigned long long> d_counters;
   std::vector<ShadeRec> mask_shades;   // directions the cached masks were swept for
-  void* ev_fused = nullptr;       // EventPairs around the fused kernels / the shading sweeps of the last run
-  void* ev_sweep = nullptr;
+  EventPairs ev_fused, ev_sweep;   // around the fused kernels / the shading sweeps of the last run
   // SWE statistics of the initial raster (first CSV row)
   double swe0_sum = 0.0, swe0_nsnow = 0.0, swe0_nvalid = 0.0;
   // runtime
   cudaStream_t stream = nullptr;
   cudaStream_t own_stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  bool ev_pending = false;
   int64_t launches = 0;
-  double last_ms = 0.0;
   LaunchInfo info{};
 };
 
 namespace {
 
 size_t rsize(const enrgy_ctx* c) { return c->precision == ENRGY_F32 ? 4 : 8; }
+
+// f(float{}) or f(double{}): the handle's precision as a type
+template <typename F>
+auto with_precision(const enrgy_ctx* c, F&& f) {
+  return c->precision == ENRGY_F32 ? f(float{}) : f(double{});
+}
+
+// terrain normals of the band for the in-kernel insolation; terrain: full raster laid out like the DEM buffer
+cudaError_t launch_normals(enrgy_ctx* c, const float* terrain) {
+  return with_precision(c, [&](auto r) {
+    using R = decltype(r);
+    return launch_terrain<R>(c->dem0, terrain, c->dem_pitch, c->rows, c->cols, c->pitch, c->band_row0, c->band_rows_pad,
+                             c->p.cell_size, (R*)c->d_nx.p, (R*)c->d_ny.p, (R*)c->d_nz.p, c->stream);
+  });
+}
+
+// the band's cells of three padded device state rasters src[q] (in the handle's precision) into the host
+// buffers dst[q] (skipped when null) as float32 (dtype 32) or float64 (64)
+int download_state(enrgy_ctx* c, int dtype, const unsigned char* const src[3], void* const dst[3]) {
+  if (dtype != 32 && dtype != 64) return fail(ENRGY_ERR_ARG, "dtype must be 32 or 64");
+  const size_t n = (size_t)c->band_rows * c->cols;
+  const size_t osz = dtype == 32 ? 4 : 8;
+  CU_TRY(c->d_stage.alloc(n * osz));
+  for (int q = 0; q < 3; ++q) {
+    if (!dst[q]) continue;
+    CU_TRY(with_precision(c, [&](auto r) {
+      using R = decltype(r);
+      return launch_unpad_state<R>((const R*)src[q], c->pitch, c->band_rows, c->cols, dtype, c->d_stage.p, c->stream);
+    }));
+    c->launches++;
+    CU_TRY(cudaMemcpyAsync(dst[q], c->d_stage.p, n * osz, cudaMemcpyDeviceToHost, c->stream));
+    CU_TRY(cudaStreamSynchronize(c->stream));
+  }
+  return ENRGY_OK;
+}
 
 int use_device(enrgy_ctx* c) {
   if (!c) return fail(ENRGY_ERR_ARG, "null context");
@@ -169,14 +245,11 @@ int upload_padded(enrgy_ctx* c, const float* src, int rows, float* dst, int rows
   return ENRGY_OK;
 }
 
-template <typename R>
-int convert_state(enrgy_ctx* c, const float* d_src32, unsigned char* dst) {
-  CU_TRY(launch_pad_convert<R>(d_src32, (R*)dst, c->band_elems, c->stream));
-  c->launches++;
-  return ENRGY_OK;
-}
+constexpr const char* kNanWhereDemValid = "%s is NaN at %llu cells where the DEM is valid; the reference would propagate NaN "
+                                          "into only some of its area means there -- not supported";
 
-int check_mask(enrgy_ctx* c, const float* d_other, const char* what, bool strict_other_valid) {
+// fails with ENRGY_ERR_MASK (nan_fmt, what, count) when d_other is NaN where the DEM of the band is valid
+int check_mask(enrgy_ctx* c, const float* d_other, const char* what, const char* nan_fmt = kNanWhereDemValid) {
   CU_TRY(c->d_counters.alloc(2));
   CU_TRY(cudaMemsetAsync(c->d_counters.p, 0, 2 * sizeof(unsigned long long), c->stream));
   CU_TRY(launch_mask_check(c->dem0, c->dem_pitch, d_other, c->pitch, c->band_row0, c->band_rows, c->cols,
@@ -185,16 +258,7 @@ int check_mask(enrgy_ctx* c, const float* d_other, const char* what, bool strict
   unsigned long long h[2];
   CU_TRY(cudaMemcpyAsync(h, c->d_counters.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
   CU_TRY(cudaStreamSynchronize(c->stream));
-  if (h[0] != 0) {
-    return fail(ENRGY_ERR_MASK,
-                "%s is NaN at %llu cells where the DEM is valid; the reference would propagate NaN "
-                "into only some of its area means there -- not supported",
-                what, h[0]);
-  }
-  if (strict_other_valid && h[1] != 0) {
-    return fail(ENRGY_ERR_MASK, "%s is valid at %llu cells where the DEM is NaN -- not supported", what,
-                h[1]);
-  }
+  if (h[0] != 0) return fail(ENRGY_ERR_MASK, nan_fmt, what, h[0]);
   return ENRGY_OK;
 }
 
@@ -298,6 +362,25 @@ void resolve_defaults(enrgy_params& p) {
   dflt(p.latent_corr, 1.0);
 }
 
+// terrain at the AWS cell and its 8 neighbours (NaN outside the raster)
+void aws_neighbourhood(const float* dem, int rows, int cols, int aws_row, int aws_col, float* nbhd /*[9]*/) {
+  for (int dr = -1; dr <= 1; ++dr)
+    for (int dc = -1; dc <= 1; ++dc) {
+      const int r = aws_row + dr, x = aws_col + dc;
+      nbhd[(dr + 1) * 3 + (dc + 1)] = (r >= 0 && r < rows && x >= 0 && x < cols) ? dem[(size_t)r * cols + x]
+                                                                            : std::numeric_limits<float>::quiet_NaN();
+    }
+}
+
+int check_forcing(int n_steps, const double* forcing) {
+  for (int i = 0; i < n_steps; ++i) {
+    const double* f = forcing + (size_t)i * ENRGY_F_COUNT;
+    if (!(f[ENRGY_F_RH] <= 1.0)) return fail(ENRGY_ERR_RANGE, "row %d: HUMID must be a 0..1 fraction here (helpers.py:74-87)", i);
+    if (!(f[ENRGY_F_DT] > 0)) return fail(ENRGY_ERR_RANGE, "row %d: time step must be > 0", i);
+  }
+  return ENRGY_OK;
+}
+
 // ---- early host pre-pass ----------------------------------------------------------------------
 // The per-step scalars depend on the forcing table, the parameters and the DEM around the AWS cell
 // only (not on the albedo / SWE rasters, unless the sub-surface model integrates the AWS cell).  So
@@ -327,8 +410,22 @@ void start_early_prepass(enrgy_ctx* c) {
   c->pre_thread = std::thread([c, in]() { c->pre_early_rc = run_prepass(in, c->pre_early, c->pre_early_err); });
 }
 
+// the fused-kernel instance of this handle's mode
+FusedVariant fused_variant(const enrgy_ctx* c, bool dump, int nm = 1, bool stats = true) {
+  FusedVariant v;
+  v.insol = c->p.insol_mode == ENRGY_INSOL_STREAMED ? kInsolStreamed : c->p.shadow ? kInsolMasked : kInsolComputed;
+  v.msm = c->p.msm_layers > 0;
+  v.dump = dump;
+  v.nm = nm;
+  v.stats = stats;
+  v.ns = c->stations_on ? kMaxStations : 1;
+  return v;
+}
+
+// arguments of a fused pass over the steps [t0, t1) of the handle's own state; masks: sunlit masks of this
+// band from the run's sunlit sub-step sub0 (the first of step t0) on
 template <typename R>
-int fill_args(enrgy_ctx* c, int t0, int t1, KernelArgs<R>& a) {
+void fill_args(enrgy_ctx* c, int t0, int t1, const unsigned* masks, int sub0, KernelArgs<R>& a) {
   a = KernelArgs<R>{};
   a.rows_full = c->rows; a.cols = c->cols; a.pitch = c->pitch;
   a.band_row0 = c->band_row0; a.band_rows = c->band_rows; a.rows_pad_full = c->rows_pad_full;
@@ -372,12 +469,10 @@ int fill_args(enrgy_ctx* c, int t0, int t1, KernelArgs<R>& a) {
   a.block_begin = b0; a.block_end = b1;
   a.t0 = t0; a.t1 = t1;
   a.tiles = c->d_tiles.p; a.n_tiles = c->n_tiles;
-  return ENRGY_OK;
-}
-
-int insol_variant(const enrgy_ctx* c) {
-  if (c->p.insol_mode == ENRGY_INSOL_STREAMED) return kInsolStreamed;
-  return c->p.shadow ? kInsolMasked : kInsolComputed;
+  a.masks = masks; a.mask_sub0 = sub0;
+  // (prefetches stop at the last sub-step of the range; at sub0 when it has none)
+  a.mask_sub_last = t1 > t0 ? std::max(c->pre.sub_first[t1 - 1] + c->pre.sub_count[t1 - 1] - 1, sub0) : sub0;
+  if (c->stations_on) fill_station_args<R>(c, a);
 }
 
 int check_run_ready(enrgy_ctx* c, int t0, int t1) {
@@ -392,57 +487,6 @@ int check_run_ready(enrgy_ctx* c, int t0, int t1) {
                 c->pot_t0, c->pot_t0 + c->pot_n, t0, t1);
   }
   return ENRGY_OK;
-}
-
-// ---- CUDA event pairs around the kernels of the last run (several chunks -> several pairs) ---------
-struct EventPairs {
-  std::vector<cudaEvent_t> ev;   // begin, end, begin, end, ...
-  int used = 0;
-  bool pending = false;
-  double last_ms = 0.0;
-  void reset() { used = 0; pending = false; }
-  cudaError_t begin(cudaStream_t s) {
-    while ((int)ev.size() < used + 2) {
-      cudaEvent_t e;
-      cudaError_t rc = cudaEventCreate(&e);
-      if (rc != cudaSuccess) return rc;
-      ev.push_back(e);
-    }
-    return cudaEventRecord(ev[used], s);
-  }
-  cudaError_t end(cudaStream_t s) {
-    cudaError_t rc = cudaEventRecord(ev[used + 1], s);
-    used += 2;
-    pending = true;
-    return rc;
-  }
-  double collect() {
-    if (pending) {
-      double tot = 0.0;
-      for (int i = 0; i + 1 < used; i += 2) {
-        float ms = 0.f;
-        if (cudaEventSynchronize(ev[i + 1]) == cudaSuccess && cudaEventElapsedTime(&ms, ev[i], ev[i + 1]) == cudaSuccess) tot += ms;
-      }
-      last_ms = tot;
-      pending = false;
-    }
-    return last_ms;
-  }
-  void destroy() {
-    for (cudaEvent_t e : ev) cudaEventDestroy(e);
-    ev.clear();
-  }
-};
-EventPairs& fused_events(enrgy_ctx* c);
-EventPairs& sweep_events(enrgy_ctx* c);
-
-EventPairs& fused_events(enrgy_ctx* c) {
-  if (!c->ev_fused) c->ev_fused = new EventPairs();
-  return *static_cast<EventPairs*>(c->ev_fused);
-}
-EventPairs& sweep_events(enrgy_ctx* c) {
-  if (!c->ev_sweep) c->ev_sweep = new EventPairs();
-  return *static_cast<EventPairs*>(c->ev_sweep);
 }
 
 // ---- shading: sunlit masks by the line sweep (shade.cu) -------------------------------------------
@@ -499,7 +543,7 @@ int sweep_range(enrgy_ctx* c, int sub0, int sub1, int n_seg, const SweepSeg* seg
       CU_TRY(cudaMemsetAsync(segs[q].ptr + (size_t)z * words, 0xFF, words * sizeof(unsigned), stream));
     }
   }
-  CU_TRY(sweep_events(c).begin(stream));
+  CU_TRY(c->ev_sweep.begin(stream));
   for (size_t k = 0; k < n_slices; ++k) {
     // (stream order: the transpose of slice k has read the temporary before slice k + 1 sweeps into it)
     const size_t r0 = std::min(row_subs.size(), k * kSweepMaxRowSubs), r1 = std::min(row_subs.size(), r0 + kSweepMaxRowSubs);
@@ -509,33 +553,32 @@ int sweep_range(enrgy_ctx* c, int sub0, int sub1, int n_seg, const SweepSeg* seg
     int n = 0;
     CU_TRY(launch_sweep(a, c->sm_count, stream, &n));
     c->launches += n;
-    c->sweep_launches += n;
   }
-  CU_TRY(sweep_events(c).end(stream));
+  CU_TRY(c->ev_sweep.end(stream));
   return ENRGY_OK;
 }
 
 // masks of [sub0, sub1) for this handle's own band in c->d_maskbuf (kept: they depend only on the
-// terrain and the sub-step directions, so later runs, ensemble members and debug views reuse them)
-int ensure_masks(enrgy_ctx* c, int sub0, int sub1, cudaStream_t stream) {
-  if (sub1 <= sub0) return ENRGY_OK;
-  bool hit = sub0 >= c->mask_sub0 && sub1 <= c->mask_sub1;
-  if (hit) {
-    for (int i = sub0; i < sub1 && hit; ++i) {
-      hit = std::memcmp(&c->mask_shades[i - c->mask_sub0], &c->pre.subs[i].shade, sizeof(ShadeRec)) == 0;
-    }
-  }
-  if (hit) return ENRGY_OK;
+// terrain and the sub-step directions, so later runs, ensemble members and debug views reuse them);
+// *masks = the mask of sub0
+int ensure_masks(enrgy_ctx* c, int sub0, int sub1, cudaStream_t stream, const unsigned** masks) {
   const size_t per = mask_words_per_sub(c, c->band_rows);
-  c->mask_sub0 = c->mask_sub1 = 0;
-  CU_TRY(c->d_maskbuf.alloc((size_t)(sub1 - sub0) * per));
-  SweepSeg sg{};
-  sg.row0 = c->band_row0; sg.rows = c->band_rows; sg.rg = c->band_rows_pad / 8; sg.words = c->pitch / 32;
-  sg.ptr = c->d_maskbuf.p;
-  if (int e = sweep_range(c, sub0, sub1, 1, &sg, stream)) return e;
-  c->mask_shades.resize(sub1 - sub0);
-  for (int i = sub0; i < sub1; ++i) c->mask_shades[i - sub0] = c->pre.subs[i].shade;
-  c->mask_sub0 = sub0; c->mask_sub1 = sub1;
+  bool hit = sub1 <= sub0 || (sub0 >= c->mask_sub0 && sub1 <= c->mask_sub1);
+  for (int i = sub0; i < sub1 && hit; ++i) {
+    hit = std::memcmp(&c->mask_shades[i - c->mask_sub0], &c->pre.subs[i].shade, sizeof(ShadeRec)) == 0;
+  }
+  if (!hit) {
+    c->mask_sub0 = c->mask_sub1 = 0;
+    CU_TRY(c->d_maskbuf.alloc((size_t)(sub1 - sub0) * per));
+    SweepSeg sg{};
+    sg.row0 = c->band_row0; sg.rows = c->band_rows; sg.rg = c->band_rows_pad / 8; sg.words = c->pitch / 32;
+    sg.ptr = c->d_maskbuf.p;
+    if (int e = sweep_range(c, sub0, sub1, 1, &sg, stream)) return e;
+    c->mask_shades.resize(sub1 - sub0);
+    for (int i = sub0; i < sub1; ++i) c->mask_shades[i - sub0] = c->pre.subs[i].shade;
+    c->mask_sub0 = sub0; c->mask_sub1 = sub1;
+  }
+  *masks = c->d_maskbuf.p + (size_t)(sub0 - c->mask_sub0) * per;
   return ENRGY_OK;
 }
 
@@ -566,47 +609,69 @@ std::vector<Chunk> plan_chunks(const enrgy_ctx* c, int t0, int t1) {
   return out;
 }
 
-// A run cut into several launches: defer_begin copies the SWE raster (stream-ordered), the launches that
-// follow leave total_snow alone, and after defer_last the next launch adds swe(start of the run) -
-// swe(end) -- exactly what a single launch over the whole range does.
-int defer_begin(enrgy_ctx* c, cudaStream_t stream) {
-  const size_t bytes = c->band_elems * rsize(c);
+// A run cut into several launches: defer_begin copies the SWE rasters at its start (stream-ordered; the
+// handle's own, or one per fused member slot), the launches that follow leave total_snow alone, and after
+// defer_last the next chunk adds swe(start of the run) - swe(end) -- exactly what a single launch over the
+// whole range does.
+int defer_begin(enrgy_ctx* c, const void* swe, size_t bytes, cudaStream_t stream) {
   CU_TRY(c->d_swe_ref.alloc(bytes));
-  CU_TRY(cudaMemcpyAsync(c->d_swe_ref.p, c->d_swe.p, bytes, cudaMemcpyDeviceToDevice, stream));
+  CU_TRY(cudaMemcpyAsync(c->d_swe_ref.p, swe, bytes, cudaMemcpyDeviceToDevice, stream));
   c->defer = 1;
   return ENRGY_OK;
 }
 void defer_last(enrgy_ctx* c) { if (c->defer == 1) c->defer = 2; }
+void defer_done(enrgy_ctx* c) { if (c->defer == 2) c->defer = 0; }
 
-// one launch of the fused kernel over [t0, t1) (+ statistics); masks: sunlit masks of this band, the
-// first one belonging to the run's sunlit sub-step number mask_sub0
-template <typename R>
-int launch_range(enrgy_ctx* c, int t0, int t1, double* d_stats, cudaStream_t stream, const unsigned* masks, int mask_sub0) {
-  KernelArgs<R> a;
-  fill_args<R>(c, t0, t1, a);
-  a.masks = masks; a.mask_sub0 = mask_sub0;
-  a.mask_sub_last = t1 > t0 ? c->pre.sub_first[t1 - 1] + c->pre.sub_count[t1 - 1] - 1 : mask_sub0;
-  if (a.mask_sub_last < mask_sub0) a.mask_sub_last = mask_sub0;
-  const int insol = insol_variant(c);
-  if (insol == kInsolMasked && masks == nullptr) return fail(ENRGY_ERR_ARG, "no sunlit masks for a run with shading");
-  LaunchInfo li;
-  const bool msm = c->p.msm_layers > 0;
-  if (c->stations_on) {
-    fill_station_args<R>(c, a);
-    CU_TRY(energy_balance_stations_grid<R>(insol, false, c->sm_count, a.cap_steps, a.cap_subs, &li));
-  } else {
-    CU_TRY(energy_balance_grid<R>(insol, msm, false, c->sm_count, a.cap_steps, a.cap_subs, &li));
+// Runs the steps [t0, t1) as run_chunk(chunk, masks): with shading in chunks whose sunlit masks fit the
+// budget (plan_chunks), each one's masks swept or found in the cache first; else as one chunk without
+// masks.  A run of several chunks defers total_snow to its last chunk; swe: the run's SWE rasters (bytes).
+template <typename F>
+int run_chunks(enrgy_ctx* c, int t0, int t1, const void* swe, size_t bytes, cudaStream_t stream, F&& run_chunk) {
+  const bool shaded = fused_variant(c, false).insol == kInsolMasked && t1 > t0;
+  const std::vector<Chunk> chunks = shaded ? plan_chunks(c, t0, t1) : std::vector<Chunk>{Chunk{t0, t1, 0, 0}};
+  if (chunks.size() > 1 && c->defer == 0) {
+    if (int e = defer_begin(c, swe, bytes, stream)) return e;
   }
-  int grid = std::min(li.grid, std::max(c->n_tiles, 1));
-  const int n = t1 - t0;
-  const size_t partial_bytes = (size_t)grid * std::max(n, 1) * (msm ? kStatsP : kStatsK) * sizeof(R);
-  CU_TRY(c->d_partials.alloc(partial_bytes));
-  CU_TRY(cudaMemsetAsync(c->d_partials.p, 0, partial_bytes, stream));
-  a.partials = (R*)c->d_partials.p;
-  if (n > 0 && !c->state_advanced) {
-    CU_TRY(launch_nan_offglacier<R>(c->dem0, c->dem_pitch, c->pitch, c->band_row0, c->band_rows, c->cols, a.swe,
-                                    a.total_snow, a.total_ice, stream));
-    c->launches++;
+  for (size_t q = 0; q < chunks.size(); ++q) {
+    const Chunk& ch = chunks[q];
+    if (q + 1 == chunks.size() && chunks.size() > 1) defer_last(c);
+    const unsigned* masks = nullptr;
+    if (shaded) {
+      if (int e = ensure_masks(c, ch.s0, ch.s1, stream, &masks)) return e;
+    }
+    if (int e = run_chunk(ch, masks)) return e;
+    defer_done(c);
+  }
+  return ENRGY_OK;
+}
+
+// the first run on new state rasters turns their off-glacier cells into NaN (model.py:258)
+template <typename R>
+int nan_offglacier(enrgy_ctx* c, cudaStream_t stream) {
+  if (c->state_advanced) return ENRGY_OK;
+  CU_TRY(launch_nan_offglacier<R>(c->dem0, c->dem_pitch, c->pitch, c->band_row0, c->band_rows, c->cols, (R*)c->d_swe.p,
+                                  (R*)c->d_ts.p, (R*)c->d_ti.p, stream));
+  c->launches++;
+  return ENRGY_OK;
+}
+
+// where the per-step statistics of one member of a fused pass go: its float64 step records, its rows
+struct StatsOut { const StepRec<double>* steps64; double* stats; };
+
+// one launch of the fused kernel variant v over a's steps; the statistics of the pass's members
+// 0 .. n_out - 1 are finalized into out[]
+template <typename R>
+int fused_pass(enrgy_ctx* c, KernelArgs<R>& a, const FusedVariant& v, const StatsOut* out, int n_out, cudaStream_t stream) {
+  LaunchInfo li;
+  CU_TRY(configure_energy_balance<R>(v, c->sm_count, a.cap_steps, a.cap_subs, &li));
+  const int grid = std::min(li.grid, std::max(c->n_tiles, 1));
+  const int n = a.t1 - a.t0;
+  const size_t partial_bytes = v.stats ? (size_t)grid * std::max(n, 1) * v.nm * (v.msm ? kStatsP : kStatsK) * sizeof(R) : 0;
+  if (v.stats) {
+    // (the launches are stream-ordered and finalize runs right behind its kernel: one buffer serves all)
+    CU_TRY(c->d_partials.alloc(partial_bytes));
+    CU_TRY(cudaMemsetAsync(c->d_partials.p, 0, partial_bytes, stream));
+    a.partials = (R*)c->d_partials.p;
   }
   // The per-CTA statistic rows are read-modify-written once per tile and time block.  In float32 mode they
   // (42 MB for a season) stay in L2 by themselves; the float64 rows (twice the size) were evicted by the
@@ -622,82 +687,75 @@ int launch_range(enrgy_ctx* c, int t0, int t1, double* d_stats, cudaStream_t str
     av.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
     CU_TRY(cudaStreamSetAttribute(stream, cudaStreamAttributeAccessPolicyWindow, &av));
   }
-  CU_TRY(fused_events(c).begin(stream));
-  if (c->stations_on) {
-    CU_TRY(launch_energy_balance_stations<R>(a, insol, false, c->sm_count, grid, &c->info, stream));
-  } else {
-    CU_TRY(launch_energy_balance<R>(a, nullptr, insol, false, c->sm_count, grid, &c->info, stream));
-  }
-  CU_TRY(fused_events(c).end(stream));
+  CU_TRY(c->ev_fused.begin(stream));
+  CU_TRY(launch_energy_balance<R>(a, v, c->sm_count, grid, &c->info, stream));
+  CU_TRY(c->ev_fused.end(stream));
   if (pin_rows) {
     cudaStreamAttrValue av{};
     av.accessPolicyWindow.num_bytes = 0;                 // window off for whatever follows on this stream
     CU_TRY(cudaStreamSetAttribute(stream, cudaStreamAttributeAccessPolicyWindow, &av));
   }
   c->launches++;
-  if (c->defer == 2) c->defer = 0;
-  if (d_stats && n > 0) {
+  for (int k = 0; k < n_out && n > 0; ++k) {
     FinalizeArgs f{};
-    f.partials = c->d_partials.p; f.n_ctas = grid; f.n_steps = n; f.t0 = t0;
-    f.n_valid = c->n_valid; f.f32_mode = c->precision == ENRGY_F32; f.msm = msm ? 1 : 0;
-    f.lwd_summed = c->stations_on ? 1 : 0;
+    f.partials = c->d_partials.p; f.n_ctas = grid; f.n_steps = n; f.t0 = a.t0;
+    f.nm = v.nm; f.member = k;
+    f.n_valid = c->n_valid; f.f32_mode = c->precision == ENRGY_F32; f.msm = v.msm ? 1 : 0;
+    f.lwd_summed = v.ns > 1 ? 1 : 0;
     for (int q = 0; q < 5; ++q) f.mom[q] = c->mom[q];
-    f.steps64 = c->d_steps64.p; f.stats = d_stats;
-    f.override_first = (t0 == 0 && !c->state_advanced) ? 1 : 0;
+    f.steps64 = out[k].steps64; f.stats = out[k].stats;
+    f.override_first = (a.t0 == 0 && !c->state_advanced) ? 1 : 0;
     f.swe0_sum = c->swe0_sum; f.swe0_nsnow = c->swe0_nsnow; f.swe0_nvalid = c->swe0_nvalid;
     CU_TRY(launch_finalize(f, stream));
     c->launches++;
   }
-  if (n > 0) c->state_advanced = true;
+  return ENRGY_OK;
+}
+
+// one fused pass of the handle's own state over [t0, t1) (+ statistics into d_stats); masks: sunlit masks
+// of this band from the run's sunlit sub-step sub0 on
+template <typename R>
+int launch_range(enrgy_ctx* c, int t0, int t1, double* d_stats, cudaStream_t stream, const unsigned* masks, int sub0) {
+  const FusedVariant v = fused_variant(c, false);
+  if (v.insol == kInsolMasked && masks == nullptr) return fail(ENRGY_ERR_ARG, "no sunlit masks for a run with shading");
+  KernelArgs<R> a;
+  fill_args<R>(c, t0, t1, masks, sub0, a);
+  if (t1 > t0) {
+    if (int e = nan_offglacier<R>(c, stream)) return e;
+  }
+  const StatsOut out{c->d_steps64.p, d_stats};
+  if (int e = fused_pass<R>(c, a, v, &out, d_stats ? 1 : 0, stream)) return e;
+  if (t1 > t0) c->state_advanced = true;
   return ENRGY_OK;
 }
 
 template <typename R>
 int run_typed(enrgy_ctx* c, int t0, int t1, double* d_stats, cudaStream_t stream) {
-  fused_events(c).reset();
-  sweep_events(c).reset();
-  if (insol_variant(c) != kInsolMasked || t1 <= t0) return launch_range<R>(c, t0, t1, d_stats, stream, nullptr, 0);
-  // with shading: sweep the sunlit masks of a chunk of steps, then run the fused kernel over it
-  const std::vector<Chunk> chunks = plan_chunks(c, t0, t1);
-  if (chunks.size() > 1 && c->defer == 0) {
-    if (int e = defer_begin(c, stream)) return e;
-  }
-  for (size_t q = 0; q < chunks.size(); ++q) {
-    const Chunk& ch = chunks[q];
-    if (q + 1 == chunks.size() && chunks.size() > 1) defer_last(c);
-    if (int e = ensure_masks(c, ch.s0, ch.s1, stream)) return e;
-    const unsigned* m = c->d_maskbuf.p + (size_t)(ch.s0 - c->mask_sub0) * mask_words_per_sub(c, c->band_rows);
-    if (int e = launch_range<R>(c, ch.t0, ch.t1, d_stats ? d_stats + (size_t)(ch.t0 - t0) * ENRGY_S_COUNT : nullptr, stream,
-                                m, ch.s0))
-      return e;
-  }
-  return ENRGY_OK;
+  c->ev_fused.reset();
+  c->ev_sweep.reset();
+  return run_chunks(c, t0, t1, c->d_swe.p, c->band_elems * sizeof(R), stream, [&](const Chunk& ch, const unsigned* masks) {
+    return launch_range<R>(c, ch.t0, ch.t1, d_stats ? d_stats + (size_t)(ch.t0 - t0) * ENRGY_S_COUNT : nullptr, stream,
+                           masks, ch.s0);
+  });
 }
 
 template <typename R>
 int dump_typed(enrgy_ctx* c, int t0, int t1, double* out) {
+  const FusedVariant v = fused_variant(c, true);
+  const int s0 = c->pre.sub_first[t0], s1 = c->pre.sub_first[t1 - 1] + c->pre.sub_count[t1 - 1];
+  const unsigned* masks = nullptr;
+  if (v.insol == kInsolMasked) {
+    if (int e = ensure_masks(c, s0, s1, c->stream, &masks)) return e;
+  }
   KernelArgs<R> a;
-  fill_args<R>(c, t0, t1, a);
-  const int insol = insol_variant(c);
+  fill_args<R>(c, t0, t1, masks, s0, a);
   const int n = t1 - t0;
   const size_t per_step = (size_t)ENRGY_D_COUNT * c->band_elems;
-  if (insol == kInsolMasked) {
-    const int s0 = c->pre.sub_first[t0], s1 = c->pre.sub_first[t1 - 1] + c->pre.sub_count[t1 - 1];
-    if (int e = ensure_masks(c, s0, s1, c->stream)) return e;
-    a.masks = c->d_maskbuf.p + (size_t)(s0 - c->mask_sub0) * mask_words_per_sub(c, c->band_rows);
-    a.mask_sub0 = s0;
-    a.mask_sub_last = std::max(s1 - 1, s0);
-  }
   CU_TRY(c->d_dump.alloc((size_t)n * per_step * sizeof(R)));
   CU_TRY(cudaMemsetAsync(c->d_dump.p, 0xFF, (size_t)n * per_step * sizeof(R), c->stream));
   a.dump = (R*)c->d_dump.p;
   a.dump_field_stride = c->band_elems;
-  if (c->stations_on) {
-    fill_station_args<R>(c, a);
-    CU_TRY(launch_energy_balance_stations<R>(a, insol, true, c->sm_count, 0, nullptr, c->stream));
-  } else {
-    CU_TRY(launch_energy_balance<R>(a, nullptr, insol, true, c->sm_count, 0, nullptr, c->stream));
-  }
+  CU_TRY(launch_energy_balance<R>(a, v, c->sm_count, 0, nullptr, c->stream));
   c->launches++;
   std::vector<R> h((size_t)n * per_step);
   CU_TRY(cudaMemcpyAsync(h.data(), c->d_dump.p, h.size() * sizeof(R), cudaMemcpyDeviceToHost, c->stream));
@@ -712,7 +770,6 @@ int dump_typed(enrgy_ctx* c, int t0, int t1, double* out) {
   return ENRGY_OK;
 }
 
-
 // ---- fused ensemble members (BASELINE config C5) ---------------------------------------------------
 struct MemberSpec { double offset, zm, zhe, alb_ice, alb_snow; };
 
@@ -723,16 +780,13 @@ int run_members_typed(enrgy_ctx* c, const std::vector<MemberSpec>& mem, const st
   const int n_members = (int)mem.size(), n = t1 - t0, T = c->n_steps;
   const int slots = (n_members + 1) / 2 * 2;                  // an odd count is padded by a copy of the last member
   const size_t be = c->band_elems, bytes = be * sizeof(R);
-  const int insol = insol_variant(c);
   // state of every member = the handle's current state
   CU_TRY(c->d_mstate.alloc((size_t)slots * 3 * bytes));
   R* const ms_swe = (R*)c->d_mstate.p;
   R* const ms_ts = ms_swe + (size_t)slots * be;
   R* const ms_ti = ms_ts + (size_t)slots * be;
-  if (n > 0 && !c->state_advanced) {
-    CU_TRY(launch_nan_offglacier<R>(c->dem0, c->dem_pitch, c->pitch, c->band_row0, c->band_rows, c->cols, (R*)c->d_swe.p,
-                                    (R*)c->d_ts.p, (R*)c->d_ti.p, stream));
-    c->launches++;
+  if (n > 0) {
+    if (int e = nan_offglacier<R>(c, stream)) return e;
   }
   for (int m = 0; m < slots; ++m) {
     CU_TRY(cudaMemcpyAsync(ms_swe + (size_t)m * be, c->d_swe.p, bytes, cudaMemcpyDeviceToDevice, stream));
@@ -770,36 +824,17 @@ int run_members_typed(enrgy_ctx* c, const std::vector<MemberSpec>& mem, const st
       CU_TRY(cudaMemcpyAsync(c->d_msteps64.p + (size_t)m * T, pres[m].steps.data(), (size_t)T * sizeof(StepRec<double>),
                              cudaMemcpyHostToDevice, stream));
   }
-  fused_events(c).reset();
-  sweep_events(c).reset();
+  c->ev_fused.reset();
+  c->ev_sweep.reset();
   // with shading the sunlit masks of a chunk of steps are swept once and serve every group
-  std::vector<Chunk> chunks;
-  if (insol == kInsolMasked && n > 0) chunks = plan_chunks(c, t0, t1);
-  else chunks.push_back(Chunk{t0, t1, 0, 0});
-  const bool cut = chunks.size() > 1;
-  if (cut) {                                            // SWE of every member at the start of the run
-    CU_TRY(c->d_swe_ref.alloc((size_t)slots * bytes));
-    CU_TRY(cudaMemcpyAsync(c->d_swe_ref.p, ms_swe, (size_t)slots * bytes, cudaMemcpyDeviceToDevice, stream));
-  }
-  LaunchInfo li4{}, li2{};
-  for (size_t q = 0; q < chunks.size(); ++q) {
-    const Chunk& ch = chunks[q];
-    const unsigned* masks = nullptr;
-    if (insol == kInsolMasked && ch.t1 > ch.t0) {
-      if (int e = ensure_masks(c, ch.s0, ch.s1, stream)) return e;
-      masks = c->d_maskbuf.p + (size_t)(ch.s0 - c->mask_sub0) * mask_words_per_sub(c, c->band_rows);
-    }
-    const int nc = ch.t1 - ch.t0;
+  const int rc = run_chunks(c, t0, t1, ms_swe, (size_t)slots * bytes, stream, [&](const Chunk& ch, const unsigned* masks) {
     for (const Group& g : groups) {
       KernelArgs<R> a;
-      fill_args<R>(c, ch.t0, ch.t1, a);
-      a.masks = masks; a.mask_sub0 = ch.s0;
-      a.mask_sub_last = nc > 0 ? std::max(c->pre.sub_first[ch.t1 - 1] + c->pre.sub_count[ch.t1 - 1] - 1, ch.s0) : ch.s0;
+      fill_args<R>(c, ch.t0, ch.t1, masks, ch.s0, a);
       a.swe = ms_swe + (size_t)g.first * be;
       a.total_snow = ms_ts + (size_t)g.first * be;
       a.total_ice = ms_ti + (size_t)g.first * be;
-      a.swe_ref = cut ? (const R*)c->d_swe_ref.p + (size_t)g.first * be : nullptr;
-      a.update_total_snow = (!cut || q + 1 == chunks.size()) ? 1 : 0;
+      if (a.swe_ref) a.swe_ref += (size_t)g.first * be;
       a.member_stride = be;
       a.member_recs = (const MemberRec<R>*)c->d_mrecs.p + (size_t)g.first * T;     // groups are stored one after the other
       for (int k = 0; k < g.nm; ++k) {
@@ -808,40 +843,15 @@ int run_members_typed(enrgy_ctx* c, const std::vector<MemberSpec>& mem, const st
         a.member_albedo_ice[k] = (R)ms.alb_ice;
         a.member_albedo_snow[k] = (R)ms.alb_snow;
       }
-      LaunchInfo& li = g.nm == 4 ? li4 : li2;
-      const bool with_stats = d_stats != nullptr;
-      if (li.grid == 0) CU_TRY(energy_balance_members_grid<R>(insol, g.nm, with_stats, c->sm_count, a.cap_steps, a.cap_subs, &li));
-      const int grid = std::min(li.grid, std::max(c->n_tiles, 1));
-      if (with_stats) {
-        const size_t partial_bytes = (size_t)grid * std::max(nc, 1) * g.nm * kStatsK * sizeof(R);
-        // (the launches are stream-ordered and finalize runs right behind its kernel: one buffer serves all)
-        CU_TRY(c->d_partials.alloc(partial_bytes));
-        CU_TRY(cudaMemsetAsync(c->d_partials.p, 0, partial_bytes, stream));
-        a.partials = (R*)c->d_partials.p;
-      }
-      CU_TRY(fused_events(c).begin(stream));
-      CU_TRY(launch_energy_balance_members<R>(a, insol, g.nm, with_stats, c->sm_count, grid, &c->info, stream));
-      CU_TRY(fused_events(c).end(stream));
-      c->launches++;
-      if (d_stats && nc > 0) {
-        for (int k = 0; k < g.nm; ++k) {
-          const int m = g.first + k;
-          if (m >= n_members) continue;                 // the padding copy
-          FinalizeArgs f{};
-          f.partials = c->d_partials.p; f.n_ctas = grid; f.n_steps = nc; f.t0 = ch.t0;
-          f.nm = g.nm; f.member = k;
-          f.n_valid = c->n_valid; f.f32_mode = c->precision == ENRGY_F32; f.msm = 0;
-          for (int z = 0; z < 5; ++z) f.mom[z] = c->mom[z];
-          f.steps64 = c->d_msteps64.p + (size_t)m * T;
-          f.stats = d_stats + ((size_t)m * n + (ch.t0 - t0)) * ENRGY_S_COUNT;
-          f.override_first = (ch.t0 == 0 && !c->state_advanced) ? 1 : 0;
-          f.swe0_sum = c->swe0_sum; f.swe0_nsnow = c->swe0_nsnow; f.swe0_nvalid = c->swe0_nvalid;
-          CU_TRY(launch_finalize(f, stream));
-          c->launches++;
-        }
-      }
+      std::vector<StatsOut> out;                        // (not for the padding copy)
+      for (int m = g.first; d_stats && m < g.first + g.nm && m < n_members; ++m)
+        out.push_back({c->d_msteps64.p + (size_t)m * T, d_stats + ((size_t)m * n + (ch.t0 - t0)) * ENRGY_S_COUNT});
+      if (int e = fused_pass<R>(c, a, fused_variant(c, false, g.nm, d_stats != nullptr), out.data(), (int)out.size(), stream))
+        return e;
     }
-  }
+    return ENRGY_OK;
+  });
+  if (rc != ENRGY_OK) return rc;
   if (totals_out) {
     // glacier-wide means of the final rasters of every member (no per-step statistics needed)
     constexpr int kBlocks = 128;
@@ -927,16 +937,6 @@ int enrgy_destroy(enrgy_ctx* c) {
   drop_early_prepass(c);
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
-  c->d_dem.release(); c->d_albedo.release(); c->d_pot.release(); c->d_tmp32.release();
-  c->d_nx.release(); c->d_ny.release(); c->d_nz.release(); c->d_swe.release(); c->d_ts.release();
-  c->d_ti.release(); c->d_dump.release(); c->d_stage.release(); c->d_steps.release(); c->d_subs.release();
-  c->d_steps64.release(); c->d_shades.release(); c->d_blocks.release(); c->d_tiles.release();
-  c->d_counts.release(); c->d_partials.release(); c->d_stats.release(); c->d_small.release();
-  c->d_mstate.release(); c->d_mrecs.release(); c->d_msteps64.release(); c->d_strecs.release();
-  c->d_counters.release(); c->d_snap.release(); c->d_layer_t.release(); c->d_terrain.release(); c->d_scan.release();
-  c->d_scan_t.release(); c->d_maskbuf.release(); c->d_masktmp.release(); c->d_sweepsubs.release(); c->d_swe_ref.release();
-  if (c->ev_fused) { fused_events(c).destroy(); delete static_cast<EventPairs*>(c->ev_fused); }
-  if (c->ev_sweep) { sweep_events(c).destroy(); delete static_cast<EventPairs*>(c->ev_sweep); }
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
   if (c->own_stream) cudaStreamDestroy(c->own_stream);
@@ -968,14 +968,7 @@ int enrgy_set_params(enrgy_ctx* c, const enrgy_params* pin) {
   c->base_albedo_ice = p.albedo_ice; c->base_albedo_snow = p.albedo_snow;
   c->band_row0 = p.band_row0;
   c->band_rows = p.band_rows;
-  {
-    const int insol = p.insol_mode == ENRGY_INSOL_STREAMED ? kInsolStreamed : (p.shadow ? kInsolMasked : kInsolComputed);
-    if (c->precision == ENRGY_F32) {
-      energy_balance_tile<float>(p.msm_layers > 0, insol, &c->tile_h, &c->tile_w);
-    } else {
-      energy_balance_tile<double>(p.msm_layers > 0, insol, &c->tile_h, &c->tile_w);
-    }
-  }
+  with_precision(c, [&](auto r) { energy_balance_tile<decltype(r)>(p.msm_layers > 0, &c->tile_h, &c->tile_w); });
   c->have_msm = false;
   c->band_rows_pad = round_up(std::max(c->band_rows, 1), 16);
   c->band_elems = (size_t)c->band_rows_pad * c->pitch;
@@ -990,13 +983,7 @@ int enrgy_set_dem(enrgy_ctx* c, const float* dem) {
   drop_early_prepass(c);
   if (c->p.aws_row < 0 || c->p.aws_row >= c->rows || c->p.aws_col < 0 || c->p.aws_col >= c->cols)
     return fail(ENRGY_ERR_ARG, "AWS cell (%d, %d) outside the %d x %d raster", c->p.aws_row, c->p.aws_col, c->rows, c->cols);
-  for (int dr = -1; dr <= 1; ++dr)
-    for (int dc = -1; dc <= 1; ++dc) {
-      const int r = c->p.aws_row + dr, x = c->p.aws_col + dc;
-      c->aws_nbhd[(dr + 1) * 3 + (dc + 1)] = (r >= 0 && r < c->rows && x >= 0 && x < c->cols)
-                                                 ? dem[(size_t)r * c->cols + x]
-                                                 : std::numeric_limits<float>::quiet_NaN();
-    }
+  aws_neighbourhood(dem, c->rows, c->cols, c->p.aws_row, c->p.aws_col, c->aws_nbhd);
   if (c->p.insol_mode == ENRGY_INSOL_COMPUTED && c->p.shadow) {
     c->h_dem.assign(dem, dem + (size_t)c->rows * c->cols);
   } else {
@@ -1068,13 +1055,10 @@ int enrgy_set_dem(enrgy_ctx* c, const float* dem) {
   {
     const int blocks = 296;
     CU_TRY(c->d_small.alloc((size_t)blocks * 5));
-    if (c->precision == ENRGY_F32) {
-      CU_TRY(launch_moments<float>(c->dem0, c->dem_pitch, c->band_row0, c->band_rows, c->cols, c->p.elev_aws,
-                                   c->d_small.p, blocks, c->stream));
-    } else {
-      CU_TRY(launch_moments<double>(c->dem0, c->dem_pitch, c->band_row0, c->band_rows, c->cols, c->p.elev_aws,
-                                    c->d_small.p, blocks, c->stream));
-    }
+    CU_TRY(with_precision(c, [&](auto r) {
+      return launch_moments<decltype(r)>(c->dem0, c->dem_pitch, c->band_row0, c->band_rows, c->cols, c->p.elev_aws,
+                                         c->d_small.p, blocks, c->stream);
+    }));
     c->launches++;
     std::vector<double> h((size_t)blocks * 5);
     CU_TRY(cudaMemcpyAsync(h.data(), c->d_small.p, h.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
@@ -1099,13 +1083,7 @@ int enrgy_set_dem(enrgy_ctx* c, const float* dem) {
     CU_TRY(c->d_nx.alloc(c->band_elems * rs));
     CU_TRY(c->d_ny.alloc(c->band_elems * rs));
     CU_TRY(c->d_nz.alloc(c->band_elems * rs));
-    if (c->precision == ENRGY_F32) {
-      CU_TRY(launch_terrain<float>(c->dem0, c->dem0, c->dem_pitch, c->rows, c->cols, c->pitch, c->band_row0, c->band_rows_pad,
-                                   c->p.cell_size, (float*)c->d_nx.p, (float*)c->d_ny.p, (float*)c->d_nz.p, c->stream));
-    } else {
-      CU_TRY(launch_terrain<double>(c->dem0, c->dem0, c->dem_pitch, c->rows, c->cols, c->pitch, c->band_row0, c->band_rows_pad,
-                                    c->p.cell_size, (double*)c->d_nx.p, (double*)c->d_ny.p, (double*)c->d_nz.p, c->stream));
-    }
+    CU_TRY(launch_normals(c, c->dem0));
     c->launches++;
   }
   CU_TRY(cudaStreamSynchronize(c->stream));
@@ -1133,33 +1111,11 @@ int enrgy_set_terrain(enrgy_ctx* c, const float* terrain) {
   CU_TRY(cudaMemcpy2DAsync(c->d_terrain.p, (size_t)c->dem_pitch * sizeof(float), terrain, (size_t)c->cols * sizeof(float),
                            (size_t)c->cols * sizeof(float), c->rows, cudaMemcpyHostToDevice, c->stream));
   // (the band's rows of the DEM are on the device in every mode; the mask check needs no more)
-  {
-    CU_TRY(c->d_counters.alloc(2));
-    CU_TRY(cudaMemsetAsync(c->d_counters.p, 0, 2 * sizeof(unsigned long long), c->stream));
-    CU_TRY(launch_mask_check(c->dem0, c->dem_pitch, c->d_terrain.p + (size_t)c->band_row0 * c->dem_pitch, c->dem_pitch,
-                             c->band_row0, c->band_rows, c->cols, c->d_counters.p, c->stream));
-    c->launches++;
-    unsigned long long h[2];
-    CU_TRY(cudaMemcpyAsync(h, c->d_counters.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
-    CU_TRY(cudaStreamSynchronize(c->stream));
-    if (h[0] != 0) return fail(ENRGY_ERR_MASK, "the terrain raster is NaN at %llu glacier cells", h[0]);
-  }
-  for (int dr = -1; dr <= 1; ++dr)
-    for (int dc = -1; dc <= 1; ++dc) {
-      const int r = c->p.aws_row + dr, x = c->p.aws_col + dc;
-      c->aws_nbhd[(dr + 1) * 3 + (dc + 1)] = (r >= 0 && r < c->rows && x >= 0 && x < c->cols)
-                                                 ? terrain[(size_t)r * c->cols + x]
-                                                 : std::numeric_limits<float>::quiet_NaN();
-    }
-  const size_t rs = rsize(c);
-  (void)rs;
-  if (c->precision == ENRGY_F32) {
-    CU_TRY(launch_terrain<float>(c->dem0, c->d_terrain.p, c->dem_pitch, c->rows, c->cols, c->pitch, c->band_row0, c->band_rows_pad,
-                                 c->p.cell_size, (float*)c->d_nx.p, (float*)c->d_ny.p, (float*)c->d_nz.p, c->stream));
-  } else {
-    CU_TRY(launch_terrain<double>(c->dem0, c->d_terrain.p, c->dem_pitch, c->rows, c->cols, c->pitch, c->band_row0, c->band_rows_pad,
-                                  c->p.cell_size, (double*)c->d_nx.p, (double*)c->d_ny.p, (double*)c->d_nz.p, c->stream));
-  }
+  if (int e = check_mask(c, c->d_terrain.p + (size_t)c->band_row0 * c->dem_pitch, "the terrain raster",
+                         "%s is NaN at %llu glacier cells"))
+    return e;
+  aws_neighbourhood(terrain, c->rows, c->cols, c->p.aws_row, c->p.aws_col, c->aws_nbhd);
+  CU_TRY(launch_normals(c, c->d_terrain.p));
   c->launches++;
   if (c->p.shadow) {
     c->h_terrain.assign(terrain, terrain + n);
@@ -1183,7 +1139,7 @@ int enrgy_set_albedo_maps(enrgy_ctx* c, int n_maps, const float* const* maps) {
     if (!maps[m]) return fail(ENRGY_ERR_ARG, "albedo map %d is null", m);
     float* dst = c->d_albedo.p + (size_t)m * c->band_elems;
     if (int e = upload_padded(c, maps[m], c->band_rows, dst, c->band_rows_pad)) return e;
-    if (int e = check_mask(c, dst, "albedo map", false)) return e;
+    if (int e = check_mask(c, dst, "albedo map")) return e;
   }
   c->n_maps = n_maps;
   {
@@ -1216,18 +1172,18 @@ int enrgy_set_swe(enrgy_ctx* c, const float* swe) {
   c->prepass_done = false;
   CU_TRY(c->d_tmp32.alloc(c->band_elems));
   if (int e = upload_padded(c, swe, c->band_rows, c->d_tmp32.p, c->band_rows_pad)) return e;
-  if (int e = check_mask(c, c->d_tmp32.p, "SWE raster", false)) return e;
+  if (int e = check_mask(c, c->d_tmp32.p, "SWE raster")) return e;
   const int blocks = 296;
   CU_TRY(c->d_small.alloc((size_t)blocks * 3));
   CU_TRY(launch_swe0_stats(c->d_tmp32.p, c->pitch, c->band_rows, c->cols, c->d_small.p, blocks, c->stream));
   c->launches++;
   std::vector<double> h((size_t)blocks * 3);
   CU_TRY(cudaMemcpyAsync(h.data(), c->d_small.p, h.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-  if (c->precision == ENRGY_F32) {
-    if (int e = convert_state<float>(c, c->d_tmp32.p, c->d_swe.p)) return e;
-  } else {
-    if (int e = convert_state<double>(c, c->d_tmp32.p, c->d_swe.p)) return e;
-  }
+  CU_TRY(with_precision(c, [&](auto r) {
+    using R = decltype(r);
+    return launch_pad_convert<R>(c->d_tmp32.p, (R*)c->d_swe.p, c->band_elems, c->stream);
+  }));
+  c->launches++;
   CU_TRY(cudaStreamSynchronize(c->stream));
   c->swe0_sum = c->swe0_nsnow = c->swe0_nvalid = 0.0;
   for (int b = 0; b < blocks; ++b) {
@@ -1245,28 +1201,20 @@ int enrgy_set_msm(enrgy_ctx* c, const double* temps, double elev) {
   if (!temps) return fail(ENRGY_ERR_ARG, "temps is null");
   const size_t rs = rsize(c);
   CU_TRY(c->d_layer_t.alloc((size_t)(nl + 1) * c->band_elems * rs));
-  if (c->precision == ENRGY_F32) {
-    CU_TRY(launch_msm_init<float>(c->dem0, c->dem_pitch, c->pitch, c->band_row0, c->band_rows_pad, nl + 1, temps,
-                                  elev, (float*)c->d_layer_t.p, c->band_elems, c->stream));
-  } else {
-    CU_TRY(launch_msm_init<double>(c->dem0, c->dem_pitch, c->pitch, c->band_row0, c->band_rows_pad, nl + 1, temps,
-                                   elev, (double*)c->d_layer_t.p, c->band_elems, c->stream));
-  }
-  c->launches++;
-  // the AWS cell's own boundary temperatures for the serial pre-pass, model.py:133-143
-  const float z = c->aws_nbhd[4];
   c->layer_t_aws.assign(nl + 1, 0.0);
-  for (int l = 0; l <= nl; ++l) {
-    double t;
-    if (c->precision == ENRGY_F32) {
-      const float d = z - (float)elev;
-      volatile float prod = d * -0.006f;
-      t = (double)((float)temps[l] + prod);
-    } else {
-      t = temps[l] + ((double)z - elev) * -0.006;
+  CU_TRY(with_precision(c, [&](auto r) {
+    using R = decltype(r);
+    // the AWS cell's own boundary temperatures for the serial pre-pass, model.py:133-143, rounded like the kernel's
+    const R d = (R)c->aws_nbhd[4] - (R)elev;
+    for (int l = 0; l <= nl; ++l) {
+      volatile R prod = d * (R)-0.006;
+      const double t = (double)((R)temps[l] + prod);
+      c->layer_t_aws[l] = t > 0 ? 0.0 : t;
     }
-    c->layer_t_aws[l] = t > 0 ? 0.0 : t;
-  }
+    return launch_msm_init<R>(c->dem0, c->dem_pitch, c->pitch, c->band_row0, c->band_rows_pad, nl + 1, temps, elev,
+                              (R*)c->d_layer_t.p, c->band_elems, c->stream);
+  }));
+  c->launches++;
   c->have_msm = true;
   c->prepass_done = false;
   return ENRGY_OK;
@@ -1325,11 +1273,7 @@ int enrgy_set_stations(enrgy_ctx* c, int n_extra, const double* row, const doubl
 int enrgy_set_forcing(enrgy_ctx* c, int n_steps, const double* forcing) {
   if (int e = use_device(c)) return e;
   if (n_steps < 0 || (n_steps > 0 && !forcing)) return fail(ENRGY_ERR_ARG, "bad forcing table");
-  for (int i = 0; i < n_steps; ++i) {
-    const double* f = forcing + (size_t)i * ENRGY_F_COUNT;
-    if (!(f[ENRGY_F_RH] <= 1.0)) return fail(ENRGY_ERR_RANGE, "row %d: HUMID must be a 0..1 fraction here (helpers.py:74-87)", i);
-    if (!(f[ENRGY_F_DT] > 0)) return fail(ENRGY_ERR_RANGE, "row %d: time step must be > 0", i);
-  }
+  if (int e = check_forcing(n_steps, forcing)) return e;
   drop_early_prepass(c);
   c->forcing.assign(forcing, forcing + (size_t)n_steps * ENRGY_F_COUNT);
   c->n_steps = n_steps;
@@ -1355,7 +1299,7 @@ int enrgy_set_insolation(enrgy_ctx* c, int t0, int n, const float* pot) {
   }
   // NaN masks: checked on the first raster of the window (the reference writes them all with one cutline)
   if (n > 0) {
-    if (int e = check_mask(c, c->d_pot.p, "insolation raster", false)) return e;
+    if (int e = check_mask(c, c->d_pot.p, "insolation raster")) return e;
   }
   CU_TRY(cudaStreamSynchronize(c->stream));
   c->pot_t0 = t0;
@@ -1400,14 +1344,15 @@ int enrgy_prepass(enrgy_ctx* c) {
     rc = run_prepass(in, c->pre, err);
   }
   if (rc != ENRGY_OK) return fail(rc, "%s", err.c_str());
-  const int urc = c->precision == ENRGY_F32 ? upload_tables<float>(c) : upload_tables<double>(c);
-  if (urc != ENRGY_OK) return urc;
-  if (c->stations_on) {
-    if ((int)c->st_series.size() != c->n_extra * c->n_steps * ENRGY_ST_COUNT)
-      return fail(ENRGY_ERR_ARG, "station series were set for another forcing table: call enrgy_set_stations after enrgy_set_forcing");
-    const int src = c->precision == ENRGY_F32 ? upload_stations<float>(c) : upload_stations<double>(c);
-    if (src != ENRGY_OK) return src;
-  }
+  if (int e = with_precision(c, [&](auto r) {
+        using R = decltype(r);
+        if (int e2 = upload_tables<R>(c)) return e2;
+        if (!c->stations_on) return (int)ENRGY_OK;
+        if ((int)c->st_series.size() != c->n_extra * c->n_steps * ENRGY_ST_COUNT)
+          return fail(ENRGY_ERR_ARG, "station series were set for another forcing table: call enrgy_set_stations after enrgy_set_forcing");
+        return upload_stations<R>(c);
+      }))
+    return e;
   c->prepass_done = true;
   return ENRGY_OK;
 }
@@ -1425,20 +1370,11 @@ int enrgy_host_prepass(const enrgy_params* pin, int precision, int rows, int col
   if (in.p.aws_row < 0 || in.p.aws_row >= rows || in.p.aws_col < 0 || in.p.aws_col >= cols)
     return fail(ENRGY_ERR_ARG, "AWS cell (%d, %d) outside the %d x %d raster", in.p.aws_row, in.p.aws_col, rows, cols);
   in.precision = precision; in.rows = rows; in.cols = cols; in.dem = dem;
-  for (int dr = -1; dr <= 1; ++dr)
-    for (int dc = -1; dc <= 1; ++dc) {
-      const int r = in.p.aws_row + dr, x = in.p.aws_col + dc;
-      in.nbhd[(dr + 1) * 3 + (dc + 1)] = (r >= 0 && r < rows && x >= 0 && x < cols) ? dem[(size_t)r * cols + x]
-                                                                                 : std::numeric_limits<float>::quiet_NaN();
-    }
+  aws_neighbourhood(dem, rows, cols, in.p.aws_row, in.p.aws_col, in.nbhd);
   in.n_steps = n_steps; in.forcing = forcing;
   std::vector<double> nan_pot(std::max(n_steps, 1), std::numeric_limits<double>::quiet_NaN());
   in.pot_aws = pot_aws ? pot_aws : nan_pot.data();
-  for (int i = 0; i < n_steps; ++i) {
-    const double* f = forcing + (size_t)i * ENRGY_F_COUNT;
-    if (!(f[ENRGY_F_RH] <= 1.0)) return fail(ENRGY_ERR_RANGE, "row %d: HUMID must be a 0..1 fraction here (helpers.py:74-87)", i);
-    if (!(f[ENRGY_F_DT] > 0)) return fail(ENRGY_ERR_RANGE, "row %d: time step must be > 0", i);
-  }
+  if (int e = check_forcing(n_steps, forcing)) return e;
   PrepassOutput out;
   std::string err;
   const int rc = run_prepass(in, out, err);
@@ -1496,7 +1432,7 @@ int enrgy_run_async(enrgy_ctx* c, int t0, int t1, double* d_stats, void* stream)
   if (int e = use_device(c)) return e;
   if (int e = check_run_ready(c, t0, t1)) return e;
   cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
-  return c->precision == ENRGY_F32 ? run_typed<float>(c, t0, t1, d_stats, s) : run_typed<double>(c, t0, t1, d_stats, s);
+  return with_precision(c, [&](auto r) { return run_typed<decltype(r)>(c, t0, t1, d_stats, s); });
 }
 
 int enrgy_run(enrgy_ctx* c, int t0, int t1, double* stats_out) {
@@ -1508,8 +1444,7 @@ int enrgy_run(enrgy_ctx* c, int t0, int t1, double* stats_out) {
     CU_TRY(c->d_stats.alloc((size_t)n * ENRGY_S_COUNT));
     d_stats = c->d_stats.p;
   }
-  const int rc = c->precision == ENRGY_F32 ? run_typed<float>(c, t0, t1, d_stats, c->stream)
-                                           : run_typed<double>(c, t0, t1, d_stats, c->stream);
+  const int rc = with_precision(c, [&](auto r) { return run_typed<decltype(r)>(c, t0, t1, d_stats, c->stream); });
   if (rc != ENRGY_OK) return rc;
   if (d_stats) CU_TRY(cudaMemcpyAsync(stats_out, d_stats, (size_t)n * ENRGY_S_COUNT * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
   CU_TRY(cudaStreamSynchronize(c->stream));
@@ -1557,18 +1492,20 @@ int enrgy_run_members(enrgy_ctx* c, int n_members, const double* albedo_offset, 
     if (c->p.albedo_const) { c->p.albedo_ice = mem[0].alb_ice; c->p.albedo_snow = mem[0].alb_snow; }
     c->albedo_offset = mem[0].offset;
     c->pre = pres[0];
-    rc = c->precision == ENRGY_F32 ? upload_tables<float>(c) : upload_tables<double>(c);
-    if (rc == ENRGY_OK) { c->prepass_done = true; rc = check_run_ready(c, t0, t1); }
     const int n = t1 - t0;
     double* d_stats = nullptr;
-    if (rc == ENRGY_OK && stats_out && n > 0) {
-      cudaError_t ce = c->d_stats.alloc((size_t)n_members * n * ENRGY_S_COUNT);
-      if (ce != cudaSuccess) rc = fail(ENRGY_ERR_CUDA, "cudaMalloc of the member statistics failed: %s", cudaGetErrorString(ce));
-      d_stats = c->d_stats.p;
-    }
-    if (rc == ENRGY_OK)
-      rc = c->precision == ENRGY_F32 ? run_members_typed<float>(c, mem, pres, t0, t1, d_stats, totals_out, c->stream)
-                                     : run_members_typed<double>(c, mem, pres, t0, t1, d_stats, totals_out, c->stream);
+    rc = with_precision(c, [&](auto r) {
+      using R = decltype(r);
+      if (int e = upload_tables<R>(c)) return e;
+      c->prepass_done = true;
+      if (int e = check_run_ready(c, t0, t1)) return e;
+      if (stats_out && n > 0) {
+        cudaError_t ce = c->d_stats.alloc((size_t)n_members * n * ENRGY_S_COUNT);
+        if (ce != cudaSuccess) return fail(ENRGY_ERR_CUDA, "cudaMalloc of the member statistics failed: %s", cudaGetErrorString(ce));
+        d_stats = c->d_stats.p;
+      }
+      return run_members_typed<R>(c, mem, pres, t0, t1, d_stats, totals_out, c->stream);
+    });
     if (rc == ENRGY_OK && d_stats) {
       cudaError_t ce = cudaMemcpyAsync(stats_out, d_stats, (size_t)n_members * n * ENRGY_S_COUNT * sizeof(double),
                                        cudaMemcpyDeviceToHost, c->stream);
@@ -1588,25 +1525,11 @@ int enrgy_run_members(enrgy_ctx* c, int n_members, const double* albedo_offset, 
 int enrgy_get_member_state(enrgy_ctx* c, int member, int dtype, void* swe, void* total_snow, void* total_ice) {
   if (int e = use_device(c)) return e;
   if (member < 0 || member >= c->members_last) return fail(ENRGY_ERR_ARG, "member %d outside the last run_members (%d members)", member, c->members_last);
-  if (dtype != 32 && dtype != 64) return fail(ENRGY_ERR_ARG, "dtype must be 32 or 64");
-  const size_t n = (size_t)c->band_rows * c->cols;
-  const size_t osz = dtype == 32 ? 4 : 8;
-  CU_TRY(c->d_stage.alloc(n * osz));
-  void* dsts[3] = {swe, total_snow, total_ice};
   const size_t be = c->band_elems * rsize(c);
-  for (int q = 0; q < 3; ++q) {
-    if (!dsts[q]) continue;
-    const unsigned char* src = c->d_mstate.p + ((size_t)q * c->member_slots + member) * be;
-    if (c->precision == ENRGY_F32) {
-      CU_TRY(launch_unpad_state<float>((const float*)src, c->pitch, c->band_rows, c->cols, dtype, c->d_stage.p, c->stream));
-    } else {
-      CU_TRY(launch_unpad_state<double>((const double*)src, c->pitch, c->band_rows, c->cols, dtype, c->d_stage.p, c->stream));
-    }
-    c->launches++;
-    CU_TRY(cudaMemcpyAsync(dsts[q], c->d_stage.p, n * osz, cudaMemcpyDeviceToHost, c->stream));
-    CU_TRY(cudaStreamSynchronize(c->stream));
-  }
-  return ENRGY_OK;
+  const unsigned char* src[3];
+  for (int q = 0; q < 3; ++q) src[q] = c->d_mstate.p + ((size_t)q * c->member_slots + member) * be;
+  void* const dst[3] = {swe, total_snow, total_ice};
+  return download_state(c, dtype, src, dst);
 }
 
 int enrgy_synchronize(enrgy_ctx* c) {
@@ -1620,23 +1543,23 @@ int enrgy_dump_steps(enrgy_ctx* c, int t0, int t1, double* out) {
   if (int e = check_run_ready(c, t0, t1)) return e;
   if (!out) return fail(ENRGY_ERR_ARG, "out is null");
   if (t1 == t0) return ENRGY_OK;
-  return c->precision == ENRGY_F32 ? dump_typed<float>(c, t0, t1, out) : dump_typed<double>(c, t0, t1, out);
+  return with_precision(c, [&](auto r) { return dump_typed<decltype(r)>(c, t0, t1, out); });
 }
 
 int enrgy_shade_masks(enrgy_ctx* c, int step, int max_sub, uint32_t* out, int* n_sub_out) {
   if (int e = use_device(c)) return e;
   if (int e = check_run_ready(c, step, step + 1)) return e;
   if (!out) return fail(ENRGY_ERR_ARG, "out is null");
-  if (insol_variant(c) != kInsolMasked) return fail(ENRGY_ERR_ARG, "shade masks need insol_mode = COMPUTED with shadow = 1");
+  if (fused_variant(c, false).insol != kInsolMasked) return fail(ENRGY_ERR_ARG, "shade masks need insol_mode = COMPUTED with shadow = 1");
   const int s0 = c->pre.sub_first[step], n_sub = c->pre.sub_count[step];
   if (n_sub > max_sub) return fail(ENRGY_ERR_ARG, "step has %d sunlit sub-steps, buffer holds %d", n_sub, max_sub);
   if (n_sub_out) *n_sub_out = n_sub;
   if (n_sub == 0) return ENRGY_OK;
-  if (int e = ensure_masks(c, s0, s0 + n_sub, c->stream)) return e;
+  const unsigned* masks = nullptr;
+  if (int e = ensure_masks(c, s0, s0 + n_sub, c->stream, &masks)) return e;
   const size_t per = mask_words_per_sub(c, c->band_rows);
   std::vector<unsigned> h((size_t)n_sub * per);
-  CU_TRY(cudaMemcpyAsync(h.data(), c->d_maskbuf.p + (size_t)(s0 - c->mask_sub0) * per, h.size() * sizeof(unsigned),
-                         cudaMemcpyDeviceToHost, c->stream));
+  CU_TRY(cudaMemcpyAsync(h.data(), masks, h.size() * sizeof(unsigned), cudaMemcpyDeviceToHost, c->stream));
   CU_TRY(cudaStreamSynchronize(c->stream));
   // device layout [sub][row / 8][word][row % 8] -> [sub][row][word]; off-glacier cells and the bits
   // beyond the last column read "sunlit"
@@ -1676,7 +1599,7 @@ int enrgy_shade_scan(enrgy_ctx* c, int sub0, int sub1, int n_seg, const int* seg
                      void* const* seg_ptr, void* stream) {
   if (int e = use_device(c)) return e;
   if (!c->have_dem || !c->prepass_done) return fail(ENRGY_ERR_ARG, "set_dem / set_forcing / prepass must precede shade_scan");
-  if (insol_variant(c) != kInsolMasked) return fail(ENRGY_ERR_ARG, "shade_scan needs insol_mode = COMPUTED with shadow = 1");
+  if (fused_variant(c, false).insol != kInsolMasked) return fail(ENRGY_ERR_ARG, "shade_scan needs insol_mode = COMPUTED with shadow = 1");
   if (sub0 < 0 || sub1 > (int)c->pre.subs.size() || sub0 > sub1) return fail(ENRGY_ERR_ARG, "sub-step range outside the run");
   if (n_seg < 1 || n_seg > kMaxSweepSegs || !seg_row0 || !seg_rows || !seg_ptr) return fail(ENRGY_ERR_ARG, "1..%d row segments", kMaxSweepSegs);
   SweepSeg segs[kMaxSweepSegs];
@@ -1687,20 +1610,23 @@ int enrgy_shade_scan(enrgy_ctx* c, int sub0, int sub1, int n_seg, const int* seg
     segs[q].rg = round_up(seg_rows[q], 16) / 8; segs[q].words = c->pitch / 32;
     segs[q].ptr = static_cast<unsigned*>(seg_ptr[q]);
   }
-  sweep_events(c).reset();
+  c->ev_sweep.reset();
   return sweep_range(c, sub0, sub1, n_seg, segs, stream ? (cudaStream_t)stream : c->stream);
 }
 
 int enrgy_run_masked(enrgy_ctx* c, int t0, int t1, const void* d_masks, double* d_stats, void* stream) {
   if (int e = use_device(c)) return e;
   if (int e = check_run_ready(c, t0, t1)) return e;
-  if (insol_variant(c) != kInsolMasked) return fail(ENRGY_ERR_ARG, "run_masked needs insol_mode = COMPUTED with shadow = 1");
+  if (fused_variant(c, false).insol != kInsolMasked) return fail(ENRGY_ERR_ARG, "run_masked needs insol_mode = COMPUTED with shadow = 1");
   if (!d_masks && t1 > t0) return fail(ENRGY_ERR_ARG, "d_masks is null");
   cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
-  fused_events(c).reset();
+  c->ev_fused.reset();
   const int sub0 = t0 < c->n_steps ? c->pre.sub_first[t0] : 0;
-  return c->precision == ENRGY_F32 ? launch_range<float>(c, t0, t1, d_stats, s, static_cast<const unsigned*>(d_masks), sub0)
-                                   : launch_range<double>(c, t0, t1, d_stats, s, static_cast<const unsigned*>(d_masks), sub0);
+  const int rc = with_precision(c, [&](auto r) {
+    return launch_range<decltype(r)>(c, t0, t1, d_stats, s, static_cast<const unsigned*>(d_masks), sub0);
+  });
+  if (rc == ENRGY_OK) defer_done(c);
+  return rc;
 }
 
 int enrgy_potential_insolation(enrgy_ctx* c, int step, double* out) {
@@ -1715,24 +1641,9 @@ int enrgy_potential_insolation(enrgy_ctx* c, int step, double* out) {
 int enrgy_get_state(enrgy_ctx* c, int dtype, void* swe, void* total_snow, void* total_ice) {
   if (int e = use_device(c)) return e;
   if (!c->have_dem) return fail(ENRGY_ERR_ARG, "no state before set_dem");
-  if (dtype != 32 && dtype != 64) return fail(ENRGY_ERR_ARG, "dtype must be 32 or 64");
-  const size_t n = (size_t)c->band_rows * c->cols;
-  const size_t osz = dtype == 32 ? 4 : 8;
-  CU_TRY(c->d_stage.alloc(n * osz));
-  void* dsts[3] = {swe, total_snow, total_ice};
-  unsigned char* srcs[3] = {c->d_swe.p, c->d_ts.p, c->d_ti.p};
-  for (int q = 0; q < 3; ++q) {
-    if (!dsts[q]) continue;
-    if (c->precision == ENRGY_F32) {
-      CU_TRY(launch_unpad_state<float>((const float*)srcs[q], c->pitch, c->band_rows, c->cols, dtype, c->d_stage.p, c->stream));
-    } else {
-      CU_TRY(launch_unpad_state<double>((const double*)srcs[q], c->pitch, c->band_rows, c->cols, dtype, c->d_stage.p, c->stream));
-    }
-    c->launches++;
-    CU_TRY(cudaMemcpyAsync(dsts[q], c->d_stage.p, n * osz, cudaMemcpyDeviceToHost, c->stream));
-    CU_TRY(cudaStreamSynchronize(c->stream));
-  }
-  return ENRGY_OK;
+  const unsigned char* const src[3] = {c->d_swe.p, c->d_ts.p, c->d_ti.p};
+  void* const dst[3] = {swe, total_snow, total_ice};
+  return download_state(c, dtype, src, dst);
 }
 
 int enrgy_set_state(enrgy_ctx* c, int dtype, const void* swe, const void* total_snow, const void* total_ice) {
@@ -1840,19 +1751,19 @@ int64_t enrgy_launch_count(enrgy_ctx* c) { return c ? c->launches : 0; }
 double enrgy_last_kernel_ms(enrgy_ctx* c) {
   if (!c) return 0.0;
   cudaSetDevice(c->device);
-  return fused_events(c).collect();
+  return c->ev_fused.collect();
 }
 
 double enrgy_last_sweep_ms(enrgy_ctx* c) {
   if (!c) return 0.0;
   cudaSetDevice(c->device);
-  return sweep_events(c).collect();
+  return c->ev_sweep.collect();
 }
 
 int enrgy_defer_snow_total(enrgy_ctx* c, int on) {
   if (int e = use_device(c)) return e;
   if (!c->have_dem) return fail(ENRGY_ERR_ARG, "no state before set_dem");
-  if (on) return defer_begin(c, c->stream);
+  if (on) return defer_begin(c, c->d_swe.p, c->band_elems * rsize(c), c->stream);
   defer_last(c);
   return ENRGY_OK;
 }

@@ -1491,15 +1491,14 @@ struct CellsPerThread {
 };
 
 template <typename R>
-void energy_balance_tile(bool msm, int insol, int* tile_h, int* tile_w) {
+void energy_balance_tile(bool msm, int* tile_h, int* tile_w) {
   const int k = msm ? CellsPerThread<R, true>::value : CellsPerThread<R, false>::value;
-  (void)insol;
   const int w = kWarpsFor<R, kInsolComputed>;
   *tile_w = 32 * warps_x(w);
   *tile_h = (w / warps_x(w)) * k;
 }
-template void energy_balance_tile<float>(bool, int, int*, int*);
-template void energy_balance_tile<double>(bool, int, int*, int*);
+template void energy_balance_tile<float>(bool, int*, int*);
+template void energy_balance_tile<double>(bool, int*, int*);
 
 // fused members: half the cells per thread (their per-member state takes the registers), the handle's
 // tile list is walked in two parts
@@ -1509,8 +1508,13 @@ struct PassShape {
   static constexpr int K = (NM > 1 || NS > 1) ? KT / 2 : KT;
 };
 
-template <typename R, int INSOL, bool MSM, bool DUMP, int NM = 1, bool STATS = true, int NS = 1>
-static cudaError_t configure(int sm_count, int cap_steps, int cap_subs, LaunchInfo* info) {
+// a FusedVariant as template arguments
+template <int INSOL, bool MSM, bool DUMP, int NM, bool STATS, int NS>
+struct Instance {};
+
+template <typename R, int INSOL, bool MSM, bool DUMP, int NM, bool STATS, int NS>
+static cudaError_t configure(Instance<INSOL, MSM, DUMP, NM, STATS, NS>, int sm_count, int cap_steps, int cap_subs,
+                             LaunchInfo* info) {
   constexpr int K = PassShape<R, MSM, NM, NS>::K, KT = PassShape<R, MSM, NM, NS>::KT;
   auto kern = energy_balance_kernel<R, K, INSOL, MSM, DUMP, NM, KT, STATS, NS>;
   const int smem = smem_plan<R>(kWarpsFor<R, INSOL>, cap_steps, cap_subs, INSOL != kInsolStreamed, MSM, NM, NS, INSOL == kInsolMasked).total;
@@ -1531,12 +1535,12 @@ static cudaError_t configure(int sm_count, int cap_steps, int cap_subs, LaunchIn
   return cudaSuccess;
 }
 
-template <typename R, int INSOL, bool MSM, bool DUMP, int NM = 1, bool STATS = true, int NS = 1>
-static cudaError_t launch_one(const KernelArgs<R>& a, int sm_count, int forced_grid, LaunchInfo* info,
-                              cudaStream_t stream) {
+template <typename R, int INSOL, bool MSM, bool DUMP, int NM, bool STATS, int NS>
+static cudaError_t launch_one(Instance<INSOL, MSM, DUMP, NM, STATS, NS> inst, const KernelArgs<R>& a, int sm_count,
+                              int forced_grid, LaunchInfo* info, cudaStream_t stream) {
   constexpr int K = PassShape<R, MSM, NM, NS>::K, KT = PassShape<R, MSM, NM, NS>::KT;
   LaunchInfo li;
-  cudaError_t e = configure<R, INSOL, MSM, DUMP, NM, STATS, NS>(sm_count, a.cap_steps, a.cap_subs, &li);
+  cudaError_t e = configure<R>(inst, sm_count, a.cap_steps, a.cap_subs, &li);
   if (e != cudaSuccess) return e;
   int grid = forced_grid > 0 ? forced_grid : li.grid;
   li.grid = grid;
@@ -1546,68 +1550,40 @@ static cudaError_t launch_one(const KernelArgs<R>& a, int sm_count, int forced_g
   return cudaGetLastError();
 }
 
-// fused ensemble members: (insol, nm, stats) -> template instance; nm = 2 or 4 members per pass
-template <typename R, typename F>
-static cudaError_t dispatch_members(int insol, int nm, bool stats, F&& f) {
-#define ENRGY_CASE(I, N, S) \
-  if (insol == I && nm == N && stats == S) \
-    return f(std::integral_constant<int, I>{}, std::integral_constant<int, N>{}, std::integral_constant<bool, S>{});
-  ENRGY_CASE(0, 2, true) ENRGY_CASE(1, 2, true) ENRGY_CASE(2, 2, true)
-  ENRGY_CASE(0, 4, true) ENRGY_CASE(1, 4, true) ENRGY_CASE(2, 4, true)
-  ENRGY_CASE(0, 2, false) ENRGY_CASE(1, 2, false) ENRGY_CASE(2, 2, false)
-  ENRGY_CASE(0, 4, false) ENRGY_CASE(1, 4, false) ENRGY_CASE(2, 4, false)
+// FusedVariant -> template instance; these are all the instances there are
+template <typename F>
+static cudaError_t dispatch(const FusedVariant& v, F&& f) {
+#define ENRGY_CASE(I, M, D, N, S, NS)                                                       \
+  if (v.insol == I && v.msm == M && v.dump == D && v.nm == N && v.stats == S && v.ns == NS) \
+    return f(Instance<I, M, D, N, S, NS>{});
+#define ENRGY_INSOLS(M, D, N, S, NS) ENRGY_CASE(0, M, D, N, S, NS) ENRGY_CASE(1, M, D, N, S, NS) ENRGY_CASE(2, M, D, N, S, NS)
+  // plain: (insol, msm, dump)
+  ENRGY_INSOLS(false, false, 1, true, 1) ENRGY_INSOLS(true, false, 1, true, 1)
+  ENRGY_INSOLS(false, true, 1, true, 1) ENRGY_INSOLS(true, true, 1, true, 1)
+  // station blend: (insol, dump)
+  ENRGY_INSOLS(false, false, 1, true, kMaxStations) ENRGY_INSOLS(false, true, 1, true, kMaxStations)
+  // fused ensemble members: (insol, nm, stats)
+  ENRGY_INSOLS(false, false, 2, true, 1) ENRGY_INSOLS(false, false, 4, true, 1)
+  ENRGY_INSOLS(false, false, 2, false, 1) ENRGY_INSOLS(false, false, 4, false, 1)
+#undef ENRGY_INSOLS
 #undef ENRGY_CASE
   return cudaErrorInvalidValue;
 }
-template <typename R>
-cudaError_t energy_balance_members_grid(int insol, int nm, bool stats, int sm_count, int cap_steps, int cap_subs,
-                                        LaunchInfo* info) {
-  return dispatch_members<R>(insol, nm, stats, [&](auto i, auto n, auto st) {
-    return configure<R, decltype(i)::value, false, false, decltype(n)::value, decltype(st)::value>(sm_count, cap_steps,
-                                                                                                    cap_subs, info);
-  });
-}
-template cudaError_t energy_balance_members_grid<float>(int, int, bool, int, int, int, LaunchInfo*);
-template cudaError_t energy_balance_members_grid<double>(int, int, bool, int, int, int, LaunchInfo*);
-template <typename R>
-cudaError_t launch_energy_balance_members(const KernelArgs<R>& a, int insol, int nm, bool stats, int sm_count,
-                                          int forced_grid, LaunchInfo* info, cudaStream_t stream) {
-  return dispatch_members<R>(insol, nm, stats, [&](auto i, auto n, auto st) {
-    return launch_one<R, decltype(i)::value, false, false, decltype(n)::value, decltype(st)::value>(a, sm_count, forced_grid,
-                                                                                                     info, stream);
-  });
-}
-template cudaError_t launch_energy_balance_members<float>(const KernelArgs<float>&, int, int, bool, int, int, LaunchInfo*, cudaStream_t);
-template cudaError_t launch_energy_balance_members<double>(const KernelArgs<double>&, int, int, bool, int, int, LaunchInfo*, cudaStream_t);
 
-// station blend (kMaxStations stations): (insol, dump) -> template instance
-template <typename R, typename F>
-static cudaError_t dispatch_stations(int insol, bool dump, F&& f) {
-#define ENRGY_CASE(I, D) \
-  if (insol == I && dump == D) return f(std::integral_constant<int, I>{}, std::integral_constant<bool, D>{});
-  ENRGY_CASE(0, false) ENRGY_CASE(1, false) ENRGY_CASE(2, false)
-  ENRGY_CASE(0, true) ENRGY_CASE(1, true) ENRGY_CASE(2, true)
-#undef ENRGY_CASE
-  return cudaErrorInvalidValue;
-}
 template <typename R>
-cudaError_t energy_balance_stations_grid(int insol, bool dump, int sm_count, int cap_steps, int cap_subs, LaunchInfo* info) {
-  return dispatch_stations<R>(insol, dump, [&](auto i, auto d) {
-    return configure<R, decltype(i)::value, false, decltype(d)::value, 1, true, kMaxStations>(sm_count, cap_steps, cap_subs, info);
-  });
+cudaError_t configure_energy_balance(const FusedVariant& v, int sm_count, int cap_steps, int cap_subs, LaunchInfo* info) {
+  return dispatch(v, [&](auto inst) { return configure<R>(inst, sm_count, cap_steps, cap_subs, info); });
 }
-template cudaError_t energy_balance_stations_grid<float>(int, bool, int, int, int, LaunchInfo*);
-template cudaError_t energy_balance_stations_grid<double>(int, bool, int, int, int, LaunchInfo*);
+template cudaError_t configure_energy_balance<float>(const FusedVariant&, int, int, int, LaunchInfo*);
+template cudaError_t configure_energy_balance<double>(const FusedVariant&, int, int, int, LaunchInfo*);
+
 template <typename R>
-cudaError_t launch_energy_balance_stations(const KernelArgs<R>& a, int insol, bool dump, int sm_count, int forced_grid,
-                                           LaunchInfo* info, cudaStream_t stream) {
-  return dispatch_stations<R>(insol, dump, [&](auto i, auto d) {
-    return launch_one<R, decltype(i)::value, false, decltype(d)::value, 1, true, kMaxStations>(a, sm_count, forced_grid, info,
-                                                                                              stream);
-  });
+cudaError_t launch_energy_balance(const KernelArgs<R>& a, const FusedVariant& v, int sm_count, int grid, LaunchInfo* info,
+                                  cudaStream_t stream) {
+  return dispatch(v, [&](auto inst) { return launch_one<R>(inst, a, sm_count, grid, info, stream); });
 }
-template cudaError_t launch_energy_balance_stations<float>(const KernelArgs<float>&, int, bool, int, int, LaunchInfo*, cudaStream_t);
-template cudaError_t launch_energy_balance_stations<double>(const KernelArgs<double>&, int, bool, int, int, LaunchInfo*, cudaStream_t);
+template cudaError_t launch_energy_balance<float>(const KernelArgs<float>&, const FusedVariant&, int, int, LaunchInfo*, cudaStream_t);
+template cudaError_t launch_energy_balance<double>(const KernelArgs<double>&, const FusedVariant&, int, int, LaunchInfo*, cudaStream_t);
 
 // glacier-wide means of the state rasters of fused members: block_out[(member * blocks + b) * 4 + {0..3}] =
 // {sum swe, sum total_snow, sum total_ice, count} over the band's glacier cells (summed on the host in
@@ -1650,43 +1626,6 @@ cudaError_t launch_member_totals(const float* dem, int dem_pitch, int pitch, int
 }
 template cudaError_t launch_member_totals<float>(const float*, int, int, int, int, int, const float*, const float*, const float*, size_t, int, double*, int, cudaStream_t);
 template cudaError_t launch_member_totals<double>(const float*, int, int, int, int, int, const double*, const double*, const double*, size_t, int, double*, int, cudaStream_t);
-
-// runtime (insol, msm, dump) -> template instance
-template <typename R, typename F>
-static cudaError_t dispatch(int insol, bool msm, bool dump, F&& f) {
-#define ENRGY_CASE(I, M, D) \
-  if (insol == I && msm == M && dump == D) return f(std::integral_constant<int, I>{}, std::integral_constant<bool, M>{}, std::integral_constant<bool, D>{});
-  ENRGY_CASE(0, false, false) ENRGY_CASE(1, false, false) ENRGY_CASE(2, false, false)
-  ENRGY_CASE(0, true, false) ENRGY_CASE(1, true, false) ENRGY_CASE(2, true, false)
-  ENRGY_CASE(0, false, true) ENRGY_CASE(1, false, true) ENRGY_CASE(2, false, true)
-  ENRGY_CASE(0, true, true) ENRGY_CASE(1, true, true) ENRGY_CASE(2, true, true)
-#undef ENRGY_CASE
-  return cudaErrorInvalidValue;
-}
-
-template <typename R>
-cudaError_t energy_balance_grid(int insol, bool msm, bool dump, int sm_count, int cap_steps, int cap_subs,
-                                LaunchInfo* info) {
-  return dispatch<R>(insol, msm, dump, [&](auto i, auto m, auto d) {
-    return configure<R, decltype(i)::value, decltype(m)::value, decltype(d)::value>(sm_count, cap_steps, cap_subs,
-                                                                                    info);
-  });
-}
-template cudaError_t energy_balance_grid<float>(int, bool, bool, int, int, int, LaunchInfo*);
-template cudaError_t energy_balance_grid<double>(int, bool, bool, int, int, int, LaunchInfo*);
-
-template <typename R>
-cudaError_t launch_energy_balance(const KernelArgs<R>& a, const void* reserved, int insol, bool dump,
-                                  int sm_count, int forced_grid, LaunchInfo* info, cudaStream_t stream) {
-  (void)reserved;
-  const bool msm = a.msm.layers > 0;
-  return dispatch<R>(insol, msm, dump, [&](auto i, auto m, auto d) {
-    return launch_one<R, decltype(i)::value, decltype(m)::value, decltype(d)::value>(a, sm_count, forced_grid,
-                                                                                     info, stream);
-  });
-}
-template cudaError_t launch_energy_balance<float>(const KernelArgs<float>&, const void*, int, bool, int, int, LaunchInfo*, cudaStream_t);
-template cudaError_t launch_energy_balance<double>(const KernelArgs<double>&, const void*, int, bool, int, int, LaunchInfo*, cudaStream_t);
 
 // initial boundary temperatures of the sub-surface model, model.py:133-143
 template <typename R>

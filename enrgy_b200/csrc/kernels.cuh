@@ -127,32 +127,29 @@ cudaError_t launch_nan_offglacier(const float* dem, int dem_pitch, int pitch, in
 struct LaunchInfo {
   int regs, smem_bytes, ctas_per_sm, grid, cells_per_thread;
 };
+// one instance of the fused kernel: insolation source, sub-surface model, dump mode, fused ensemble members
+// (nm = 2 or 4, no sub-surface model; stats = false: no per-step statistics, a.partials unused) and blended
+// weather stations (ns = kMaxStations, no sub-surface model, no fused members)
+struct FusedVariant {
+  int insol = kInsolStreamed;
+  bool msm = false, dump = false;
+  int nm = 1;
+  bool stats = true;
+  int ns = 1;
+};
+// the variant's kernel attributes and its full grid (cudaErrorInvalidValue: no such instance)
 template <typename R>
-cudaError_t launch_energy_balance(const KernelArgs<R>& a, const void* reserved, int insol, bool dump,
-                                  int sm_count, int forced_grid, LaunchInfo* info, cudaStream_t stream);
-// nm = 2 or 4 ensemble members fused into one pass (no sub-surface model); stats = false: no per-step
-// statistics (a.partials unused)
+cudaError_t configure_energy_balance(const FusedVariant& v, int sm_count, int cap_steps, int cap_subs, LaunchInfo* info);
+// grid > 0: that many CTAs, else the full grid; info (may be null) receives the launch's attributes
 template <typename R>
-cudaError_t launch_energy_balance_members(const KernelArgs<R>& a, int insol, int nm, bool stats, int sm_count,
-                                          int forced_grid, LaunchInfo* info, cudaStream_t stream);
-template <typename R>
-cudaError_t energy_balance_members_grid(int insol, int nm, bool stats, int sm_count, int cap_steps, int cap_subs,
-                                        LaunchInfo* info);
-// up to kMaxStations weather stations blended per cell (no sub-surface model, no fused members)
-template <typename R>
-cudaError_t launch_energy_balance_stations(const KernelArgs<R>& a, int insol, bool dump, int sm_count, int forced_grid,
-                                           LaunchInfo* info, cudaStream_t stream);
-template <typename R>
-cudaError_t energy_balance_stations_grid(int insol, bool dump, int sm_count, int cap_steps, int cap_subs, LaunchInfo* info);
+cudaError_t launch_energy_balance(const KernelArgs<R>& a, const FusedVariant& v, int sm_count, int grid, LaunchInfo* info,
+                                  cudaStream_t stream);
 template <typename R>
 cudaError_t launch_member_totals(const float* dem, int dem_pitch, int pitch, int band_row0, int band_rows, int cols,
                                  const R* swe, const R* tsn, const R* tic, size_t member_stride, int n_members,
                                  double* block_out /*[n_members][blocks][4]*/, int blocks, cudaStream_t stream);
 template <typename R>
-void energy_balance_tile(bool msm, int insol, int* tile_h, int* tile_w);
-template <typename R>
-cudaError_t energy_balance_grid(int insol, bool msm, bool dump, int sm_count, int cap_steps, int cap_subs,
-                                LaunchInfo* info);
+void energy_balance_tile(bool msm, int* tile_h, int* tile_w);
 // initial boundary temperatures: min(0, t_point[l] + (dem - elev) * -0.006), model.py:133-143
 template <typename R>
 cudaError_t launch_msm_init(const float* dem, int dem_pitch, int pitch, int band_row0, int band_rows_pad,
