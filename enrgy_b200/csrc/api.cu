@@ -395,6 +395,14 @@ void fill_prepass_input(enrgy_ctx* c, PrepassInput& in) {
   std::memcpy(in.nbhd, c->aws_nbhd, sizeof(in.nbhd));
   in.pot_aws = c->pot_aws.data();
   in.alb_aws = c->alb_aws; in.swe_aws = c->swe_aws; in.layer_t_aws = c->layer_t_aws;
+  if (c->stations_on) {
+    in.n_extra = c->n_extra;
+    std::memcpy(in.st_row, c->st_row, sizeof(in.st_row));
+    std::memcpy(in.st_col, c->st_col, sizeof(in.st_col));
+    std::memcpy(in.st_elev, c->st_elev, sizeof(in.st_elev));
+    in.st_series = c->st_series.data();
+    in.cloud_k = c->cloud_k;
+  }
 }
 void drop_early_prepass(enrgy_ctx* c) {
   if (c->pre_thread.joinable()) c->pre_thread.join();
@@ -480,7 +488,6 @@ int check_run_ready(enrgy_ctx* c, int t0, int t1) {
   if (t0 < 0 || t1 > c->n_steps || t0 > t1) return fail(ENRGY_ERR_ARG, "step range [%d, %d) outside [0, %d)", t0, t1, c->n_steps);
   if (!c->p.albedo_const && c->n_maps == 0) return fail(ENRGY_ERR_ARG, "albedo maps not set");
   if (c->p.msm_layers > 0 && !c->have_msm) return fail(ENRGY_ERR_ARG, "enrgy_set_msm must precede run when msm_layers > 0");
-  if (c->stations_on && c->p.msm_layers > 0) return fail(ENRGY_ERR_ARG, "the station blend does not run with the sub-surface model");
   if (c->p.insol_mode == ENRGY_INSOL_STREAMED && t1 > t0 &&
       (t0 < c->pot_t0 || t1 > c->pot_t0 + c->pot_n)) {
     return fail(ENRGY_ERR_ARG, "insolation rasters resident for steps [%d, %d), run asks [%d, %d)",
@@ -1329,6 +1336,9 @@ int enrgy_prepass(enrgy_ctx* c) {
   if (c->p.msm_layers > 0 && !c->have_msm) return fail(ENRGY_ERR_ARG, "enrgy_set_msm must precede prepass when msm_layers > 0");
   if (c->p.msm_layers > 0 && !c->p.albedo_const && (int)c->alb_aws.size() != c->n_maps)
     return fail(ENRGY_ERR_ARG, "the AWS cell lies outside this handle's row band: its albedo/SWE are needed for the sub-surface pre-pass");
+  // (before the pre-pass: with the sub-surface model it reads the series)
+  if (c->stations_on && (int)c->st_series.size() != c->n_extra * c->n_steps * ENRGY_ST_COUNT)
+    return fail(ENRGY_ERR_ARG, "station series were set for another forcing table: call enrgy_set_stations after enrgy_set_forcing");
   int rc;
   std::string err;
   if (c->pre_thread.joinable()) {          // started by enrgy_set_forcing, inputs unchanged since
@@ -1347,10 +1357,7 @@ int enrgy_prepass(enrgy_ctx* c) {
   if (int e = with_precision(c, [&](auto r) {
         using R = decltype(r);
         if (int e2 = upload_tables<R>(c)) return e2;
-        if (!c->stations_on) return (int)ENRGY_OK;
-        if ((int)c->st_series.size() != c->n_extra * c->n_steps * ENRGY_ST_COUNT)
-          return fail(ENRGY_ERR_ARG, "station series were set for another forcing table: call enrgy_set_stations after enrgy_set_forcing");
-        return upload_stations<R>(c);
+        return c->stations_on ? upload_stations<R>(c) : (int)ENRGY_OK;
       }))
     return e;
   c->prepass_done = true;

@@ -604,14 +604,15 @@ constexpr int kMaskAhead = ENRGY_MASK_AHEAD;   // sunlit masks are prefetched th
 // oracle/enrgy_oracle.py "several weather stations"): inverse-squared-distance weights and the weights
 // folded with the vapour-pressure reduction live in registers per cell, the stations' per-step values are
 // staged like the AWS records; unused stations carry weight zero.  The shortwave is attenuated by the
-// cloud field relative to the primary station (Beer-Lambert, one exp per cell-step).
+// cloud field relative to the primary station (Beer-Lambert, one exp per cell-step).  With the sub-surface
+// model the blended T, p and e drive the surface terms and the conduction step like the AWS values do.
 template <typename R, int K, int INSOL, bool MSM, bool DUMP, int NM = 1, int KT = K, bool STATS = true, int NS = 1>
 __global__ void __launch_bounds__(32 * kWarpsFor<R, INSOL>, NM > 2 ? ENRGY_MINB_MEMBERS : sizeof(R) == 4 ? ENRGY_MINB32 : ENRGY_MINB64)
 energy_balance_kernel(const KernelArgs<R> a) {
   static_assert(NM == 1 || (!MSM && !DUMP), "fused members: no sub-surface model, no dump");
   static_assert(KT % K == 0, "a patch is walked in whole parts");
   static_assert(STATS || NM > 1, "only fused members run without statistics");
-  static_assert(NS == 1 || (NM == 1 && !MSM), "station blend: no fused members, no sub-surface model");
+  static_assert(NS == 1 || NM == 1, "station blend: no fused members");
   constexpr int W = kWarpsFor<R, INSOL>;           // warps per CTA
   constexpr int WX = warps_x(W), WY = W / WX;      // patches of a tile: WX across, WY down
   constexpr int NT = 32 * W;                       // threads per CTA
@@ -1500,12 +1501,13 @@ void energy_balance_tile(bool msm, int* tile_h, int* tile_w) {
 template void energy_balance_tile<float>(bool, int*, int*);
 template void energy_balance_tile<double>(bool, int*, int*);
 
-// fused members: half the cells per thread (their per-member state takes the registers), the handle's
-// tile list is walked in two parts
+// fused members and the station blend: half the cells per thread (their per-member state / station weights
+// take the registers), the handle's tile list is walked in two parts -- but never less than one pair (the
+// float64 sub-surface model already runs one pair, KT = 2)
 template <typename R, bool MSM, int NM, int NS = 1>
 struct PassShape {
   static constexpr int KT = CellsPerThread<R, MSM>::value;
-  static constexpr int K = (NM > 1 || NS > 1) ? KT / 2 : KT;
+  static constexpr int K = (NM > 1 || NS > 1) ? (KT / 2 > 2 ? KT / 2 : 2) : KT;
 };
 
 // a FusedVariant as template arguments
@@ -1560,8 +1562,9 @@ static cudaError_t dispatch(const FusedVariant& v, F&& f) {
   // plain: (insol, msm, dump)
   ENRGY_INSOLS(false, false, 1, true, 1) ENRGY_INSOLS(true, false, 1, true, 1)
   ENRGY_INSOLS(false, true, 1, true, 1) ENRGY_INSOLS(true, true, 1, true, 1)
-  // station blend: (insol, dump)
+  // station blend: (insol, msm, dump)
   ENRGY_INSOLS(false, false, 1, true, kMaxStations) ENRGY_INSOLS(false, true, 1, true, kMaxStations)
+  ENRGY_INSOLS(true, false, 1, true, kMaxStations) ENRGY_INSOLS(true, true, 1, true, kMaxStations)
   // fused ensemble members: (insol, nm, stats)
   ENRGY_INSOLS(false, false, 2, true, 1) ENRGY_INSOLS(false, false, 4, true, 1)
   ENRGY_INSOLS(false, false, 2, false, 1) ENRGY_INSOLS(false, false, 4, false, 1)

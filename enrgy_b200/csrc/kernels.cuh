@@ -129,7 +129,7 @@ struct LaunchInfo {
 };
 // one instance of the fused kernel: insolation source, sub-surface model, dump mode, fused ensemble members
 // (nm = 2 or 4, no sub-surface model; stats = false: no per-step statistics, a.partials unused) and blended
-// weather stations (ns = kMaxStations, no sub-surface model, no fused members)
+// weather stations (ns = kMaxStations, no fused members); 36 combinations per precision exist
 struct FusedVariant {
   int insol = kInsolStreamed;
   bool msm = false, dump = false;

@@ -221,6 +221,27 @@ int run_prepass(const PrepassInput& in, PrepassOutput& out, std::string& err) {
   double swe_cell = in.swe_aws;
   const double delta_cell = (double)z_aws - p.elev_aws;
   const double pw_cell = std::pow(10.0, -delta_cell / kVapourScale);
+  // Station blend with the sub-surface model: the AWS cell's integration must see the blended meteorology
+  // of that cell, as every other cell does (oracle/enrgy_oracle.py "several weather stations"; station 0 is
+  // the primary AWS at the cell itself).  w: the cell's weights, v: the weights folded with the
+  // vapour-pressure reduction, d_blend: sum_k w_k (z - z_k).
+  const bool station_blend = msm && in.n_extra > 0;
+  const int n_st = 1 + in.n_extra;
+  double st_w[kMaxStations] = {}, st_v[kMaxStations] = {}, d_blend = 0.0;
+  if (station_blend) {
+    double q[kMaxStations], tot = 0.0;
+    for (int k = 0; k < n_st; ++k) {
+      const double dr = k ? (double)p.aws_row - in.st_row[k] : 0.0, dc = k ? (double)p.aws_col - in.st_col[k] : 0.0;
+      q[k] = 1.0 / (dr * dr + dc * dc + 0.25);
+      tot = k ? tot + q[k] : q[k];
+    }
+    for (int k = 0; k < n_st; ++k) {
+      const double dz = (double)z_aws - (k ? in.st_elev[k] : p.elev_aws);
+      st_w[k] = q[k] / tot;
+      d_blend = k ? d_blend + st_w[k] * dz : st_w[k] * dz;
+      st_v[k] = st_w[k] * std::pow(10.0, -dz / kVapourScale);
+    }
+  }
 
   for (int i = 0; i < T; ++i) {
     const double* f = in.forcing + (size_t)i * ENRGY_F_COUNT;
@@ -373,16 +394,36 @@ int run_prepass(const PrepassInput& in, PrepassOutput& out, std::string& err) {
     }
     s.c_sw = 3.6 * 1000000 / dt * factor;
 
+    // meteorology of the distributed pass at the AWS cell: the AWS values reduced to the cell's elevation,
+    // or their blend with the extra stations (above)
+    double t_air_c = t_air + delta_cell * f[ENRGY_F_LAPSE];
+    double p_c = p_hpa + delta_cell * kPressureLapse;
+    double e_c = e_aws * pw_cell;
+    double cloud_fac = 1.0;                        // Beer-Lambert factor of the shortwave
+    if (station_blend) {
+      const double n0 = f[ENRGY_F_CLOUD];
+      double mix_t = st_w[0] * t_air, mix_p = st_w[0] * p_hpa, mix_n = 0.0;
+      e_c = e_aws * st_v[0];
+      for (int k = 1; k < n_st; ++k) {
+        const double* v = in.st_series + ((size_t)(k - 1) * T + i) * ENRGY_ST_COUNT;
+        const double tk = v[ENRGY_ST_T_AIR], pk = v[ENRGY_ST_PRESSURE];
+        mix_t = mix_t + st_w[k] * tk;
+        mix_p = mix_p + st_w[k] * pk;
+        e_c = e_c + v[ENRGY_ST_RH] * sat_vapour_pressure(tk + 273.15, pk * 100) * st_v[k];
+        mix_n = mix_n + st_w[k] * (v[ENRGY_ST_CLOUD] - n0);
+      }
+      t_air_c = mix_t + d_blend * f[ENRGY_F_LAPSE];
+      p_c = mix_p + d_blend * kPressureLapse;
+      if (!std::isnan(in.cloud_k)) cloud_fac = std::exp(-in.cloud_k * mix_n);
+    }
     // turbulent fluxes of the distributed pass at the AWS cell itself (debug_point_output, model.py:441-448)
-    const double t_air_c = t_air + delta_cell * f[ENRGY_F_LAPSE];
     const double tz_c = t_air_c + 273.15;
     const double tsk = ts_aws_c + 273.15;
-    const double p_c = p_hpa + delta_cell * kPressureLapse;
     const double r_rt = 1.0 / (kRair * tz_c);
     const double sens = (s.c_sens * p_c) * (r_rt * (tz_c - tsk));
     const double f_p = 1.0016 + 3.15 * 1e-6 * p_c - 0.074 / p_c;
     const double es = 611.2 * std::exp((17.62 * ts_aws_c) / (243.12 + ts_aws_c)) * f_p;
-    const double lat = (s.c_lat * r_rt) * (e_aws * pw_cell - es);
+    const double lat = (s.c_lat * r_rt) * (e_c - es);
     pt[ENRGY_P_SENS_AWS] = sens;
     pt[ENRGY_P_LAT_AWS] = lat;
     if (msm) {
@@ -401,7 +442,7 @@ int run_prepass(const PrepassInput& in, PrepassOutput& out, std::string& err) {
         const double blend = x0 + s.alb_w * (x1 - x0);
         alb = has_snow ? (s.snow_alb >= 0 ? s.snow_alb : blend) : std::min(blend, p.max_ice_albedo);
       }
-      const double rs = pot_aws_kwh * s.c_sw * (1.0 - alb);
+      const double rs = pot_aws_kwh * s.c_sw * cloud_fac * (1.0 - alb);
       const double atmo = rs + lwd - lwu + sens + lat;
       double sd = swe_cell / p.snow_density;
       double grad_prev = 0.0, mf = 0.0;

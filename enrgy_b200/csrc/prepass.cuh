@@ -41,6 +41,13 @@ struct PrepassInput {
   std::vector<double> alb_aws;
   double swe_aws = 0.0;
   std::vector<double> layer_t_aws;
+  // station blend (enrgy_set_stations): extra station k = 1 .. n_extra at (st_row, st_col) of the full raster
+  // in cell units, elevation st_elev, series [n_extra][n_steps][ENRGY_ST_COUNT]; with the sub-surface model
+  // the AWS cell is integrated in the blended meteorology of that cell
+  int n_extra = 0;
+  double st_row[kMaxStations] = {}, st_col[kMaxStations] = {}, st_elev[kMaxStations] = {};
+  const double* st_series = nullptr;
+  double cloud_k = NAN;    // NaN: no cloud attenuation
 };
 
 struct PrepassOutput {

@@ -215,8 +215,13 @@ int enrgy_get_member_state(enrgy_ctx* ctx, int member, int dtype, void* swe, voi
  * Monin-Obukhov solve, exchange coefficients, lapse rate, longwave cloudiness and the observed shortwave
  * factor stay the primary station's.  cloud_k >= 0: incoming shortwave times exp(-cloud_k * (blended
  * cloudiness - the primary station's)); NaN: off.  n_extra = 0 runs the blend with the primary station
- * alone (same rasters as a plain run); n_extra < 0 switches it off.  Not with the sub-surface model or
- * enrgy_run_members.  At most 3 extra stations. */
+ * alone (same rasters as a plain run); n_extra < 0 switches it off.  With the sub-surface model the blended
+ * T, p and e (and the cloud factor) drive the surface temperature terms and the conduction step of every
+ * cell, and the pre-pass integrates the AWS cell in the blend at that cell (its weights give the extra
+ * stations a share there too): enrgy_get_point_layers, ENRGY_P_TSURF_AWS and ENRGY_P_SENS_AWS /
+ * ENRGY_P_LAT_AWS then describe the AWS cell of the blended field.  (Without the sub-surface model the two
+ * flux columns keep the AWS values reduced to the cell's elevation.)  Not with enrgy_run_members.  At most
+ * 3 extra stations. */
 enum enrgy_station_col {
   ENRGY_ST_T_AIR = 0,   /* T_AIR [deg C] */
   ENRGY_ST_PRESSURE,    /* PRESSURE [hPa] */
@@ -246,7 +251,8 @@ int enrgy_set_insolation_aws(enrgy_ctx* ctx, int t0, int n, const double* pot_aw
 int enrgy_prepass(enrgy_ctx* ctx);
 int enrgy_get_point_scalars(enrgy_ctx* ctx, double* out /* [n_steps][ENRGY_P_COUNT] */);
 /* sub-surface model: boundary temperatures of the AWS cell BEFORE each row's update (the columns
- * debug_point_output prints when msm_xy is the AWS cell, model.py:421-426); out [n_steps][msm_layers + 1] */
+ * debug_point_output prints when msm_xy is the AWS cell, model.py:421-426); out [n_steps][msm_layers + 1].
+ * With the station blend: the cell integrated in the blended meteorology (enrgy_set_stations). */
 int enrgy_get_point_layers(enrgy_ctx* ctx, double* out);
 /* the AWS cell's own values for a handle whose row band does not hold it (the sub-surface pre-pass
  * integrates that cell on every rank): its albedo-map values and initial SWE.  Call after

@@ -3,6 +3,7 @@
 the shading path on a fixed raster.  Not part of the bench contract.
 
   python scripts/measure_modes.py streamed|msm
+  python scripts/measure_modes.py msm --stations 3 [--no-msm]    (the station blend of bench.py's C4)
   torchrun ... scripts/measure_modes.py strong --n 8192 --t 96
 """
 import argparse
@@ -42,6 +43,9 @@ def main():
     ap.add_argument("--sequential", action="store_true", help="ensemble: one run per member instead of fused passes")
     ap.add_argument("--shadow", action="store_true", help="ensemble: with topographic shading")
     ap.add_argument("--nostats", action="store_true", help="ensemble: fused passes without per-step statistics")
+    ap.add_argument("--stations", type=int, default=0,
+                    help="msm: blend this many extra weather stations (bench.py C4's spots, cloud_k = 0.7)")
+    ap.add_argument("--no-msm", action="store_true", help="msm: the same run without the sub-surface model")
     a = ap.parse_args()
     prec = _lib.F32 if a.dtype == "f32" else _lib.F64
     if a.mode == "ensemble":
@@ -101,16 +105,25 @@ def main():
         eng = Engine(a.n, a.n, precision=prec)
         kw = dict(cell_size=10.0, elev_aws=case.elev_aws, aws_row=case.aws_rc[0], aws_col=case.aws_rc[1],
                   sensor_z=1.6, zm=1e-3, z_h_or_e=1e-4, emissivity=0.98, lat=case.lat, lon=case.lon)
+        msm = a.mode == "msm" and not a.no_msm
         if a.mode == "streamed":
             eng.set_params(insol_mode=_lib.INSOL_STREAMED, **kw)
         else:
-            eng.set_params(insol_mode=_lib.INSOL_COMPUTED, msm_depths=[0.1, 0.1, 0.3, 0.5, 0.5, 0.5, 3.0], **kw)
+            eng.set_params(insol_mode=_lib.INSOL_COMPUTED, msm_depths=[0.1, 0.1, 0.3, 0.5, 0.5, 0.5, 3.0] if msm else None, **kw)
         eng.set_dem(dem)
-        if a.mode == "msm":
+        if msm:
             eng.set_msm([-6.9, -6.93, -7.025, -7.31, -6.93, -7.12, -7.0, -5.57], 275.0)
         eng.set_albedo_maps([case.albedo_maps[k] for k in keys])
         eng.set_swe(case.swe)
         eng.set_forcing(build_forcing(case.aws_rows, keys))
+        if a.mode == "msm" and a.stations > 0:
+            from enrgy_b200.forcing import build_station_series
+            from enrgy_b200.synthetic import make_station_rows
+            spots = [(0.2 * a.n, 0.3 * a.n, 150.0, 41), (0.75 * a.n, 0.7 * a.n, -80.0, 42), (0.5 * a.n, 0.9 * a.n, 60.0, 43)]
+            spots = spots[:a.stations]
+            eng.set_stations([(r, c, case.elev_aws + dz) for (r, c, dz, _) in spots],
+                             [build_station_series(make_station_rows(case, case.elev_aws + dz, seed=sd)) for (_, _, dz, sd) in spots],
+                             cloud_k=0.7)
         if a.mode == "streamed":
             rng = np.random.default_rng(0)
             field = (0.6 + 0.4 * rng.random((a.n, a.n))).astype(np.float32)
@@ -127,7 +140,8 @@ def main():
         eng.prepass()
         ms = timed(eng, a.t)
         cells = float(a.n) * a.n * a.t
-        print(json.dumps({"mode": a.mode, "dtype": a.dtype, "n": a.n, "t": a.t, "kernel_ms": ms,
+        print(json.dumps({"mode": a.mode, "msm": msm, "stations": a.stations if a.mode == "msm" else 0,
+                          "dtype": a.dtype, "n": a.n, "t": a.t, "kernel_ms": ms,
                           "cell_steps_per_s": cells / (ms * 1e-3), "kernel": eng.kernel_info(),
                           "streamed_GBps": (cells * 0.70 * 4 / (ms * 1e-3) / 1e9) if a.mode == "streamed" else None}))
         eng.close()
