@@ -565,12 +565,22 @@ int sweep_range(enrgy_ctx* c, int sub0, int sub1, int n_seg, const SweepSeg* seg
   return ENRGY_OK;
 }
 
+// sunlit sub-steps of the steps [t0, t1) (0 for an empty range and for rows where the sun stays down)
+int sunlit_subs(const enrgy_ctx* c, int t0, int t1) {
+  return t1 > t0 ? c->pre.sub_first[t1 - 1] + c->pre.sub_count[t1 - 1] - c->pre.sub_first[t0] : 0;
+}
+
 // masks of [sub0, sub1) for this handle's own band in c->d_maskbuf (kept: they depend only on the
 // terrain and the sub-step directions, so later runs, ensemble members and debug views reuse them);
-// *masks = the mask of sub0
+// *masks = the mask of sub0, or null for an empty range (the kernel reads no mask in a row without a
+// sunlit sub-step)
 int ensure_masks(enrgy_ctx* c, int sub0, int sub1, cudaStream_t stream, const unsigned** masks) {
+  if (sub1 <= sub0) {
+    *masks = nullptr;
+    return ENRGY_OK;
+  }
   const size_t per = mask_words_per_sub(c, c->band_rows);
-  bool hit = sub1 <= sub0 || (sub0 >= c->mask_sub0 && sub1 <= c->mask_sub1);
+  bool hit = sub0 >= c->mask_sub0 && sub1 <= c->mask_sub1;
   for (int i = sub0; i < sub1 && hit; ++i) {
     hit = std::memcmp(&c->mask_shades[i - c->mask_sub0], &c->pre.subs[i].shade, sizeof(ShadeRec)) == 0;
   }
@@ -720,11 +730,13 @@ int fused_pass(enrgy_ctx* c, KernelArgs<R>& a, const FusedVariant& v, const Stat
 }
 
 // one fused pass of the handle's own state over [t0, t1) (+ statistics into d_stats); masks: sunlit masks
-// of this band from the run's sunlit sub-step sub0 on
+// of this band from the run's sunlit sub-step sub0 on (may be null when the range has no sunlit sub-step:
+// the kernel reads a mask only inside a sub-step)
 template <typename R>
 int launch_range(enrgy_ctx* c, int t0, int t1, double* d_stats, cudaStream_t stream, const unsigned* masks, int sub0) {
   const FusedVariant v = fused_variant(c, false);
-  if (v.insol == kInsolMasked && masks == nullptr) return fail(ENRGY_ERR_ARG, "no sunlit masks for a run with shading");
+  if (v.insol == kInsolMasked && masks == nullptr && sunlit_subs(c, t0, t1) > 0)
+    return fail(ENRGY_ERR_ARG, "no sunlit masks for a run with shading");
   KernelArgs<R> a;
   fill_args<R>(c, t0, t1, masks, sub0, a);
   if (t1 > t0) {
@@ -1625,7 +1637,7 @@ int enrgy_run_masked(enrgy_ctx* c, int t0, int t1, const void* d_masks, double* 
   if (int e = use_device(c)) return e;
   if (int e = check_run_ready(c, t0, t1)) return e;
   if (fused_variant(c, false).insol != kInsolMasked) return fail(ENRGY_ERR_ARG, "run_masked needs insol_mode = COMPUTED with shadow = 1");
-  if (!d_masks && t1 > t0) return fail(ENRGY_ERR_ARG, "d_masks is null");
+  if (!d_masks && sunlit_subs(c, t0, t1) > 0) return fail(ENRGY_ERR_ARG, "d_masks is null");
   cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
   c->ev_fused.reset();
   const int sub0 = t0 < c->n_steps ? c->pre.sub_first[t0] : 0;

@@ -230,7 +230,8 @@ class ShardedShading:
             sl = self._recv(k % 2, recv_words)
             self.subs_last_scan = b - a           # (last_sweep_ms() of the engine times the last scan only)
             if world == 1:
-                eng.shade_scan(a, b, [(self.bands[0][0], self.bands[0][1], sl["recv"].data_ptr())], sp)
+                if b > a:
+                    eng.shade_scan(a, b, [(self.bands[0][0], self.bands[0][1], sl["recv"].data_ptr())], sp)
             elif self.exchange == "p2p":
                 # all ranks are done with this slot (fused kernels of chunk k - 2) before anybody writes into it
                 if k >= 2:
@@ -302,7 +303,9 @@ class ShardedShading:
             if len(plan) > 1 and k == len(plan) - 1:
                 eng.defer_snow_total(False)
             stats_ptr = None if d_stats_ptr is None else d_stats_ptr + 8 * _lib.S_COUNT * (c0 - t0)
-            eng.run_masked(c0, c1, sl["recv"].data_ptr(), stats_ptr, sp)
+            # a chunk without a sunlit sub-step (polar night) needs no masks
+            s0, s1 = eng.sub_range(c0, c1)
+            eng.run_masked(c0, c1, sl["recv"].data_ptr() if s1 > s0 else None, stats_ptr, sp)
 
 
 def allreduce_stats(stats):

@@ -136,7 +136,9 @@ typedef struct enrgy_params {
   double lon_deg;
   double solar_const;    /* NaN = 1367 */
   double transmittance;  /* NaN = 0.70 */
-  double hour_step;      /* NaN = 0.25 h */
+  double hour_step;      /* NaN = 0.25 h.  Computed insolation: a step may hold at most 255 SUNLIT
+                            sub-steps of this length, so dt <= 63.75 h always passes at the default;
+                            enrgy_prepass refuses a step with more with ENRGY_ERR_RANGE */
   /* --- sub-surface model (model.py:126-149, msm.py:31-107) --- */
   int32_t msm_layers;    /* 0 = off; else number of layer THICKNESSES (boundaries = layers + 1) */
   int32_t _pad2;
@@ -303,7 +305,8 @@ int64_t enrgy_mask_words(enrgy_ctx* ctx, int rows);
 int enrgy_shade_scan(enrgy_ctx* ctx, int sub0, int sub1, int n_seg, const int* seg_row0, const int* seg_rows,
                      void* const* seg_ptr, void* stream);
 /* the fused kernels over the rows [t0, t1) with the caller's masks of this handle's band for exactly
- * the sub-steps of enrgy_sub_range(t0, t1); otherwise like enrgy_run_async */
+ * the sub-steps of enrgy_sub_range(t0, t1); otherwise like enrgy_run_async.  d_masks may be NULL when
+ * those rows have no sunlit sub-step (polar night): no mask is read then. */
 int enrgy_run_masked(enrgy_ctx* ctx, int t0, int t1, const void* d_masks, double* d_stats, void* stream);
 /* A run the CALLER cuts into several enrgy_run_masked / enrgy_run_async calls (chunks of rows): call with
  * on = 1 before the first and with on = 0 before the last.  The snow-melt total is then formed once, as

@@ -173,8 +173,10 @@ def oracle_band_sums(ora, rows, valid):
     return out
 
 
-def compare_run(case, f64, pot=None, computed=False, shadow=False, band=None, ora=None, **kw):
+def compare_run(case, f64, pot=None, computed=False, shadow=False, band=None, ora=None, skip=(), **kw):
     """Runs oracle and engine; returns dict of worst relative errors.
+    skip: (row, field) pairs of the per-step flux rasters left out of res[field]; their worst error is
+    res["skipped"] (only with skip).
     band = (row0, rows): the engine runs that row band; its rasters are compared with those rows of the
     whole-raster oracle and its statistics with the oracle's float64 sums over them ("band_sums"; the
     glacier-wide means only exist for the whole raster).  ora: run_oracle's result for these inputs, for
@@ -200,12 +202,16 @@ def compare_run(case, f64, pot=None, computed=False, shadow=False, band=None, or
         # very case (SURVEY 8c): the as-shipped reference deviates from its float64-injected self by a few
         # 1e-3 W m-2 in the melt flux (the gate carries the cold content of the surface layer, which integrates
         # the float32 round-off of every earlier step).  1e-4 x 5 W m-2 = 5e-4 W m-2 must not be looser than that.
-        ora64 = run_oracle(case, oracle_insolation(case, pot, computed, shadow, True), True, **kw)
-        own_gap = max(float(np.nanmax(np.abs(np.asarray(a["mf"], dtype=np.float64) - b["mf"])))
-                      for a, b in zip(ora["rows"], ora64["rows"]))
-        assert 1e-4 * msm_floor <= own_gap, ("the float32 melt-flux bound is looser than the reference's own float32 "
-                                             "error on this case", own_gap)
+        # Where nothing melts (a cold regime), mf is exactly 0 in both runs and the reference has no such
+        # error to measure: the bound then rests on the cases that melt.
+        if any(np.nanmax(r["mf"]) > 0 for r in ora["rows"]):
+            ora64 = run_oracle(case, oracle_insolation(case, pot, computed, shadow, True), True, **kw)
+            own_gap = max(float(np.nanmax(np.abs(np.asarray(a["mf"], dtype=np.float64) - b["mf"])))
+                          for a, b in zip(ora["rows"], ora64["rows"]))
+            assert 1e-4 * msm_floor <= own_gap, ("the float32 melt-flux bound is looser than the reference's own "
+                                                 "float32 error on this case", own_gap)
     res = {}
+    skipped = 0.0
     off = np.isnan(case.dem)[rows]
     for name in FLUX_FIELDS:
         idx = _lib.DUMP_NAMES.index(name)
@@ -226,8 +232,14 @@ def compare_run(case, f64, pot=None, computed=False, shadow=False, band=None, or
                 # step's fluxes (3e-5 W m-2 per term, in the as-shipped reference too): the
                 # per-step melt flux agrees to ~5e-4 W m-2, the melt TOTALS to 1e-4 relative.
                 floor = msm_floor
-            worst = max(worst, max_rel_err(dump[i, idx], ref, floor))
+            e = max_rel_err(dump[i, idx], ref, floor)
+            if (i, name) in skip:
+                skipped = max(skipped, e)
+            else:
+                worst = max(worst, e)
         res[name] = worst
+    if skip:
+        res["skipped"] = skipped
     worst = 0.0
     for i in range(n):
         ref = np.array(ora["rows"][i]["albedo"], dtype=np.float64)[rows]
@@ -260,6 +272,17 @@ def compare_run(case, f64, pot=None, computed=False, shadow=False, band=None, or
         floors[[_lib.S_NSNOW, _lib.S_NSWE, _lib.S_NVALID]] = 0.5
         scale = np.maximum(s_o[:, [_lib.S_NVALID]], 1.0)
         res["band_sums"] = float(np.max(np.abs(stats - s_o) / np.maximum(np.abs(s_o), floors * scale)))
-    res["L"] = float(np.max(np.abs(point[:, _lib.P_L] - [r["L"] for r in ora["rows"]])
-                            / np.abs([r["L"] for r in ora["rows"]])))
+    res["L"] = l_rel_err(point[:, _lib.P_L], [r["L"] for r in ora["rows"]])
     return res
+
+
+def l_rel_err(got, ref):
+    """Worst relative error of the Monin-Obukhov lengths.  A neutral row (air at the surface temperature:
+    Qh = 0) has L = +inf; an infinity matched by the same infinity counts as exact, any other value
+    against it as an infinite error."""
+    got = np.asarray(got, dtype=np.float64)
+    ref = np.asarray(ref, dtype=np.float64)
+    with np.errstate(invalid="ignore"):
+        e = np.abs(got - ref) / np.abs(ref)
+    e = np.where(np.isinf(ref) & (got == ref), 0.0, e)
+    return float(np.max(np.where(np.isnan(e), np.inf, e)))

@@ -132,14 +132,22 @@ def test_insolation_tables_match_oracle():
         assert max(abs(r["dc_fix"]), abs(r["dr_fix"])) == 65536
 
 
+REGIME_VARIANTS = ["polar_night", "polar_dawn", "polar_dusk", "cold_unstable", "extremes", "irregular_time"]
+
+
 @pytest.mark.parametrize("f64", [True, False])
-@pytest.mark.parametrize("variant", ["default", "andreas", "gradient_calm"])
+@pytest.mark.parametrize("variant", ["default", "andreas", "gradient_calm"] + REGIME_VARIANTS)
 def test_host_prepass_matches_oracle(f64, variant):
     """The library's host pre-pass (C++: Monin-Obukhov solve, CH, shortwave factor; csrc/prepass.cu,
     reached through enrgy_host_prepass WITHOUT a device) against the oracle's per-row scalars, which are
-    the reference's own (turbo.py:88-137, model.py:500-530).  No GPU, no kernel: host logic only."""
+    the reference's own (turbo.py:88-137, model.py:500-530).  No GPU, no kernel: host logic only.
+    The weather regimes of tests/regimes.py (with their insolation, dark where the sun is down) reach the
+    unstable branch of the Monin-Obukhov solve and the neutral row (L = +inf), gales, calm air, dry and
+    saturated air, a station at 600-660 hPa and rows of 10 min to 63.75 h."""
     from enrgy_b200.engine import host_prepass
+    from oracle import insolation_oracle as I
     from tests import parity as P
+    from tests import regimes as G
     kw = {}
     case_kw = {}
     if variant == "andreas":
@@ -147,8 +155,12 @@ def test_host_prepass_matches_oracle(f64, variant):
     if variant == "gradient_calm":
         case_kw = dict(with_gradient=True, calm_every=5)     # GRADIENT column, WIND_SPEED 0 -> 0.1
         kw = dict(temp_lapse_rate="GRADIENT")
-    case = make_case(48, 30, w=56, seed=17, **case_kw)
-    pot = P.random_insolation(case, 30)
+    if variant in REGIME_VARIANTS:
+        case = G.make_regime_case(variant)
+        pot = I.insolation_series(case, shadow=False).astype(np.float32)
+    else:
+        case = make_case(48, 30, w=56, seed=17, **case_kw)
+        pot = P.random_insolation(case, 30)
     ora = P.run_oracle(case, pot, f64, **kw)
     alb = P.clipped_albedo(case, np.float32)
     table = build_forcing(case.aws_rows, list(alb), temp_lapse_rate=kw.get("temp_lapse_rate", -0.006))
@@ -159,8 +171,15 @@ def test_host_prepass_matches_oracle(f64, variant):
                          insol_mode=_lib.INSOL_STREAMED, lat=case.lat, lon=case.lon)
     L_ref = np.array([r["L"] for r in ora["rows"]])
     f_ref = np.array([r["factor"] for r in ora["rows"]])
-    assert np.max(np.abs(point[:, _lib.P_L] - L_ref) / np.abs(L_ref)) < (1e-9 if f64 else 1e-5)
+    assert P.l_rel_err(point[:, _lib.P_L], L_ref) < (1e-9 if f64 else 1e-5)
     assert np.max(np.abs(point[:, _lib.P_SW_FACTOR] - f_ref) / np.maximum(np.abs(f_ref), 1e-12)) < (1e-12 if f64 else 1e-6)
+    if variant == "cold_unstable":
+        # both branches and the neutral row really occur
+        assert (L_ref < 0).sum() >= 10 and (L_ref > 0).any() and np.isposinf(L_ref).sum() >= 3
+    if variant == "polar_night":
+        assert np.all(f_ref == 1.0)                          # potential insolation 0 -> factor 1
+    if variant in ("polar_dawn", "polar_dusk"):
+        assert f_ref.max() > 3.0                             # a faint SWD over a sun at the horizon
 
 
 def test_host_prepass_computed_insolation_and_errors():
@@ -171,6 +190,7 @@ def test_host_prepass_computed_insolation_and_errors():
     from enrgy_b200._lib import EnrgyError
     from oracle import insolation_oracle as I
     from oracle.enrgy_oracle import time_step_seconds
+    from datetime import datetime, timedelta
     case = make_case(64, 12, w=72, seed=19)
     table = build_forcing(case.aws_rows, list(case.albedo_maps))
     base = dict(cell_size=case.cell, elev_aws=case.elev_aws, aws_row=case.aws_rc[0], aws_col=case.aws_rc[1],
@@ -185,6 +205,42 @@ def test_host_prepass_computed_insolation_and_errors():
             assert abs(got_kwh - want) <= 1e-9 * max(abs(want), 1e-6), (shadow, i)
             n_sub = len(I.substep_table(I.to_unix(row["DATE"]), dt, case.lat, case.lon, case.cell))
             assert int(point[i, _lib.P_NSUB]) == n_sub
+    # dark, dawn and irregular rows: 0 .. 255 sunlit sub-steps, partial last sub-steps
+    from tests import regimes as G
+    for name in ("polar_night", "polar_dawn", "polar_dusk", "irregular_time"):
+        rc = G.make_regime_case(name)
+        t_rc = build_forcing(rc.aws_rows, list(rc.albedo_maps))
+        b_rc = dict(base, elev_aws=rc.elev_aws, aws_row=rc.aws_rc[0], aws_col=rc.aws_rc[1])
+        counts = []
+        for shadow in (False, True):
+            point = host_prepass(rc.dem, t_rc, shadow=shadow, **b_rc)
+            for i, row in enumerate(rc.aws_rows):
+                dt = time_step_seconds(rc.aws_rows, i)
+                n_sub = len(I.substep_table(I.to_unix(row["DATE"]), dt, rc.lat, rc.lon, rc.cell))
+                assert int(point[i, _lib.P_NSUB]) == n_sub, (name, i)
+                if not shadow:
+                    counts.append(n_sub)
+                want = I.potential_insolation(rc.dem, rc.cell, rc.lat, rc.lon, I.to_unix(row["DATE"]), dt,
+                                              shadow=shadow)[rc.aws_rc]
+                assert abs(point[i, _lib.P_POT_AWS] * dt / 3.6e6 - want) <= 1e-9 * max(abs(want), 1e-6), (name, shadow, i)
+        if name == "polar_night":
+            assert set(counts) == {0}
+        elif name == "irregular_time":
+            assert {0, 1, 4, 12, 28, 255} <= set(counts)
+        else:
+            assert 0 in counts and 4 in counts and any(0 < k < 4 for k in counts)
+    # at most 255 sunlit sub-steps in one row: 63.75 h of midnight sun pass, 64 h are refused
+    for hours, ok in ((63.75, True), (64.0, False)):
+        rows = G.make_regime_case("irregular_time").aws_rows[:2]
+        rows = [dict(rows[0], DATE="20220620 00:00:00"),
+                dict(rows[1], DATE=(datetime(2022, 6, 20) + timedelta(hours=hours)).strftime("%Y%m%d %H:%M:%S"))]
+        t_b = build_forcing(rows, ["20220601", "20220701"])
+        if ok:
+            assert list(host_prepass(case.dem, t_b, **base)[:, _lib.P_NSUB]) == [255, 255]
+        else:
+            with pytest.raises(EnrgyError) as err:
+                host_prepass(case.dem, t_b, **base)
+            assert err.value.code == _lib.ERR_RANGE
     with pytest.raises(EnrgyError):
         host_prepass(case.dem, table, **dict(base, aws_row=999))
     bad = table.copy()
