@@ -24,6 +24,9 @@ namespace {
 
 thread_local std::string g_err;
 
+// largest raster side (rows or columns) accepted, include/enrgy_b200.h:enrgy_create and DESIGN.md §3
+constexpr int kMaxSide = 1 << 20;
+
 int fail(int code, const char* fmt, ...) {
   char buf[1024];
   va_list ap;
@@ -913,8 +916,8 @@ int enrgy_device_count(void) {
 int enrgy_create(int device, int rows, int cols, int precision, enrgy_ctx** out) {
   if (!out) return fail(ENRGY_ERR_ARG, "out is null");
   *out = nullptr;
-  if (rows <= 0 || cols <= 0 || rows > 32767 || cols > 32767)
-    return fail(ENRGY_ERR_ARG, "raster %d x %d outside 1..32767", rows, cols);
+  if (rows <= 0 || cols <= 0 || rows > kMaxSide || cols > kMaxSide)
+    return fail(ENRGY_ERR_ARG, "raster %d x %d outside 1..%d", rows, cols, kMaxSide);
   if (precision != ENRGY_F32 && precision != ENRGY_F64) return fail(ENRGY_ERR_ARG, "precision must be 32 or 64");
   const int n = enrgy_device_count();
   if (n <= 0) return fail(ENRGY_ERR_NODEVICE, "no CUDA device visible; enrgy_b200 has no CPU fallback");
@@ -1380,7 +1383,8 @@ int enrgy_host_prepass(const enrgy_params* pin, int precision, int rows, int col
                        const double* forcing, const double* pot_aws, double* point_out) {
   if (!pin || !dem || (n_steps > 0 && (!forcing || !point_out))) return fail(ENRGY_ERR_ARG, "null argument");
   if (precision != ENRGY_F32 && precision != ENRGY_F64) return fail(ENRGY_ERR_ARG, "precision must be 32 or 64");
-  if (rows <= 0 || cols <= 0 || n_steps < 0) return fail(ENRGY_ERR_ARG, "bad sizes");
+  if (rows <= 0 || cols <= 0 || rows > kMaxSide || cols > kMaxSide || n_steps < 0)
+    return fail(ENRGY_ERR_ARG, "bad sizes: raster %d x %d (1..%d a side), %d steps", rows, cols, kMaxSide, n_steps);
   PrepassInput in;
   in.p = *pin;
   resolve_defaults(in.p);

@@ -131,7 +131,9 @@ ENRGY_HD void line_geometry(int dc_fix, int dr_fix, bool* row_type, int* sigma, 
   if (*row_type) { *sigma = dr_fix > 0 ? 1 : -1; *dfix = dc_fix; }
   else { *sigma = dc_fix > 0 ? 1 : -1; *dfix = dr_fix; }
 }
-ENRGY_HD int shear_q16(int u, int dfix) { return (u * dfix + 32768) >> 16; }
+// sh(u) = round(u * dfix / 2^16).  The product is 64-bit: |dfix| <= 65536 and |u| < 2^20 (rasters up
+// to 2^20 cells a side) reach 2^36; the result, at most |u|, fits an int.
+ENRGY_HD int shear_q16(int u, int dfix) { return (int)(((long long)u * dfix + 32768) >> 16); }
 
 // time block = consecutive steps whose records and sub-steps fit the smem staging buffers
 struct TimeBlock {

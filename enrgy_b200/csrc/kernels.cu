@@ -258,43 +258,44 @@ __global__ void terrain_kernel(const float* __restrict__ dem, const float* __res
   // uncropped DEM (reference model.py:469 -> saga_lighting.py:42), so slopes at the glacier margin see
   // their real neighbours
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  const int rb = blockIdx.y;
-  if (c >= pitch || rb >= band_rows_pad) return;
-  const int r = rb + band_row0;
-  const size_t o = (size_t)rb * pitch + c;
+  if (c >= pitch) return;
   const float qnan = __int_as_float(0x7fc00000);
   auto at = [&](int rr, int cc) -> float {
     if (rr < 0 || rr >= rows_full || cc < 0 || cc >= cols) return qnan;
     return terr[(size_t)rr * dem_pitch + cc];
   };
-  const bool glacier = r < rows_full && c < cols && dem[(size_t)r * dem_pitch + c] == dem[(size_t)r * dem_pitch + c];
-  const float zf = glacier ? at(r, c) : qnan;
-  if (!(zf == zf)) {
-    nx[o] = (R)qnan; ny[o] = (R)qnan; nz[o] = (R)qnan;
-    return;
+  for (int rb = blockIdx.y; rb < band_rows_pad; rb += gridDim.y) {
+    const int r = rb + band_row0;
+    const size_t o = (size_t)rb * pitch + c;
+    const bool glacier = r < rows_full && c < cols && dem[(size_t)r * dem_pitch + c] == dem[(size_t)r * dem_pitch + c];
+    const float zf = glacier ? at(r, c) : qnan;
+    if (!(zf == zf)) {
+      nx[o] = (R)qnan; ny[o] = (R)qnan; nz[o] = (R)qnan;
+      continue;
+    }
+    const R z = (R)zf;
+    auto one_sided = [&](float a, float b) -> R {
+      if (a == a) return (R)a - z;
+      if (b == b) return z - (R)b;
+      return (R)0;
+    };
+    const float zn = at(r - 1, c), zs = at(r + 1, c), ze = at(r, c + 1), zw = at(r, c - 1);
+    const R gy = (one_sided(zn, zs) - one_sided(zs, zn)) * inv2cell;
+    const R gx = (one_sided(ze, zw) - one_sided(zw, ze)) * inv2cell;
+    // stored as (nx/nz, ny/nz, nz) = (-gx, -gy, nz): cos(incidence) = nz * (u + px*e + py*n), which
+    // costs the time loop two FMAs per sub-step instead of three
+    const R inv = Num<R>::rsqrt_((R)1 + gx * gx + gy * gy);
+    nx[o] = -gx;
+    ny[o] = -gy;
+    nz[o] = inv;
   }
-  const R z = (R)zf;
-  auto one_sided = [&](float a, float b) -> R {
-    if (a == a) return (R)a - z;
-    if (b == b) return z - (R)b;
-    return (R)0;
-  };
-  const float zn = at(r - 1, c), zs = at(r + 1, c), ze = at(r, c + 1), zw = at(r, c - 1);
-  const R gy = (one_sided(zn, zs) - one_sided(zs, zn)) * inv2cell;
-  const R gx = (one_sided(ze, zw) - one_sided(zw, ze)) * inv2cell;
-  // stored as (nx/nz, ny/nz, nz) = (-gx, -gy, nz): cos(incidence) = nz * (u + px*e + py*n), which
-  // costs the time loop two FMAs per sub-step instead of three
-  const R inv = Num<R>::rsqrt_((R)1 + gx * gx + gy * gy);
-  nx[o] = -gx;
-  ny[o] = -gy;
-  nz[o] = inv;
 }
 
 template <typename R>
 cudaError_t launch_terrain(const float* dem, const float* terr, int dem_pitch, int rows_full, int cols, int pitch,
                            int band_row0, int band_rows_pad, double cell, R* nx, R* ny, R* nz,
                            cudaStream_t stream) {
-  dim3 grid((pitch + 255) / 256, band_rows_pad);
+  dim3 grid((pitch + 255) / 256, grid_rows(band_rows_pad));
   terrain_kernel<R><<<grid, 256, 0, stream>>>(dem, terr, dem_pitch, rows_full, cols, pitch, band_row0, band_rows_pad,
                                               (R)(1.0 / (2.0 * cell)), nx, ny, nz);
   return cudaGetLastError();
@@ -306,31 +307,35 @@ template cudaError_t launch_terrain<double>(const float*, const float*, int, int
 __global__ void tile_scan_kernel(const float* __restrict__ dem, int pitch, int band_row0,
                                  int band_rows, int cols, int tile_h, int tile_w, int tiles_c,
                                  int* __restrict__ counts) {
-  const int tr = blockIdx.y, tc = blockIdx.x;
-  int n = 0;
-  for (int i = threadIdx.x; i < tile_h * tile_w; i += blockDim.x) {
-    const int rb = tr * tile_h + i / tile_w;
-    const int c = tc * tile_w + i % tile_w;
-    if (rb < band_rows && c < cols) {
-      const float z = dem[(size_t)(rb + band_row0) * pitch + c];
-      n += (z == z) ? 1 : 0;
-    }
-  }
-  n = __reduce_add_sync(0xffffffffu, n);
+  const int tc = blockIdx.x;
+  const int tiles_r = (band_rows + tile_h - 1) / tile_h;
   __shared__ int s[32];
-  if ((threadIdx.x & 31) == 0) s[threadIdx.x >> 5] = n;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int tot = 0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) tot += s[w];
-    counts[tr * tiles_c + tc] = tot;
+  for (int tr = blockIdx.y; tr < tiles_r; tr += gridDim.y) {
+    int n = 0;
+    for (int i = threadIdx.x; i < tile_h * tile_w; i += blockDim.x) {
+      const int rb = tr * tile_h + i / tile_w;
+      const int c = tc * tile_w + i % tile_w;
+      if (rb < band_rows && c < cols) {
+        const float z = dem[(size_t)(rb + band_row0) * pitch + c];
+        n += (z == z) ? 1 : 0;
+      }
+    }
+    n = __reduce_add_sync(0xffffffffu, n);
+    if ((threadIdx.x & 31) == 0) s[threadIdx.x >> 5] = n;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      int tot = 0;
+      for (int w = 0; w < (int)(blockDim.x >> 5); ++w) tot += s[w];
+      counts[(size_t)tr * tiles_c + tc] = tot;
+    }
+    __syncthreads();                    // s is refilled by the next row of tiles
   }
 }
 cudaError_t launch_tile_scan(const float* dem, int pitch, int band_row0, int band_rows, int cols,
                              int tile_h, int tile_w, int tiles_r, int tiles_c, int* counts,
                              cudaStream_t stream) {
-  tile_scan_kernel<<<dim3(tiles_c, tiles_r), 256, 0, stream>>>(dem, pitch, band_row0, band_rows, cols,
-                                                               tile_h, tile_w, tiles_c, counts);
+  tile_scan_kernel<<<dim3(tiles_c, grid_rows(tiles_r)), 256, 0, stream>>>(dem, pitch, band_row0, band_rows, cols,
+                                                                           tile_h, tile_w, tiles_c, counts);
   return cudaGetLastError();
 }
 
@@ -1623,6 +1628,7 @@ template <typename R>
 cudaError_t launch_member_totals(const float* dem, int dem_pitch, int pitch, int band_row0, int band_rows, int cols,
                                  const R* swe, const R* tsn, const R* tic, size_t member_stride, int n_members,
                                  double* block_out, int blocks, cudaStream_t stream) {
+  // grid.y = members (<= kMaxFusedMembers); the cells are a grid-stride loop, so no dimension grows with the raster
   member_totals_kernel<R><<<dim3(blocks, n_members), kThreads, 0, stream>>>(dem, dem_pitch, pitch, band_row0, band_rows, cols,
                                                                            swe, tsn, tic, member_stride, block_out);
   return cudaGetLastError();
@@ -1636,24 +1642,25 @@ __global__ void msm_init_kernel(const float* __restrict__ dem, int dem_pitch, in
                                 int band_rows_pad, int n_bounds, const R* __restrict__ t_point, R elev,
                                 R* __restrict__ layer_t, size_t layer_stride) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  const int rb = blockIdx.y;
-  if (c >= pitch || rb >= band_rows_pad) return;
-  const float z = dem[(size_t)(rb + band_row0) * dem_pitch + c];
-  const size_t o = (size_t)rb * pitch + c;
+  if (c >= pitch) return;
   const R qnan = (R)__int_as_float(0x7fc00000);
-  for (int l = 0; l < n_bounds; ++l) {
-    R t = qnan;
-    if (z == z) {
-      // value + (dem - elev) * -0.006, rounded product and rounded sum like NumPy
-      const R d = (R)z - elev;
-      if (sizeof(R) == 4) {
-        t = (R)__fadd_rn((float)t_point[l], __fmul_rn((float)d, -0.006f));
-      } else {
-        t = (R)__dadd_rn((double)t_point[l], __dmul_rn((double)d, -0.006));
+  for (int rb = blockIdx.y; rb < band_rows_pad; rb += gridDim.y) {
+    const float z = dem[(size_t)(rb + band_row0) * dem_pitch + c];
+    const size_t o = (size_t)rb * pitch + c;
+    for (int l = 0; l < n_bounds; ++l) {
+      R t = qnan;
+      if (z == z) {
+        // value + (dem - elev) * -0.006, rounded product and rounded sum like NumPy
+        const R d = (R)z - elev;
+        if (sizeof(R) == 4) {
+          t = (R)__fadd_rn((float)t_point[l], __fmul_rn((float)d, -0.006f));
+        } else {
+          t = (R)__dadd_rn((double)t_point[l], __dmul_rn((double)d, -0.006));
+        }
+        if (t > (R)0) t = (R)0;             // ice temperature is limited by the melting point
       }
-      if (t > (R)0) t = (R)0;             // ice temperature is limited by the melting point
+      layer_t[(size_t)l * layer_stride + o] = t;
     }
-    layer_t[(size_t)l * layer_stride + o] = t;
   }
 }
 template <typename R>
@@ -1667,7 +1674,7 @@ cudaError_t launch_msm_init(const float* dem, int dem_pitch, int pitch, int band
   if (e != cudaSuccess) return e;
   e = cudaMemcpyAsync(d, h, sizeof(R) * n_bounds, cudaMemcpyHostToDevice, stream);
   if (e == cudaSuccess) {
-    dim3 grid((pitch + 255) / 256, band_rows_pad);
+    dim3 grid((pitch + 255) / 256, grid_rows(band_rows_pad));
     msm_init_kernel<R><<<grid, 256, 0, stream>>>(dem, dem_pitch, pitch, band_row0, band_rows_pad, n_bounds, d,
                                                  (R)elev, layer_t, layer_stride);
     e = cudaGetLastError();
@@ -1830,7 +1837,8 @@ __global__ void finalize_stats_kernel(const FinalizeArgs f) {
 
 cudaError_t launch_finalize(const FinalizeArgs& f, cudaStream_t stream) {
   if (f.n_steps <= 0) return cudaSuccess;
-  finalize_stats_kernel<<<(f.n_steps + 3) / 4, 128, 0, stream>>>(f);      // four steps (warps) per block
+  // four steps (warps) per block; a 1-D grid over the steps, independent of the raster size
+  finalize_stats_kernel<<<(f.n_steps + 3) / 4, 128, 0, stream>>>(f);
   return cudaGetLastError();
 }
 

@@ -99,6 +99,12 @@ struct FinalizeArgs {
 };
 
 // launch helpers (defined in kernels.cu); all asynchronous on `stream`
+//
+// CUDA caps grid.y and grid.z at 65535.  Set-up kernels that give a grid row to each raster row (or row
+// tile) launch at most kMaxGridY of them and stride over the rest, so any raster of up to 2^20 rows
+// (enrgy_create) launches; below kMaxGridY rows the launch is one grid row per raster row as before.
+constexpr int kMaxGridY = 65535;
+inline int grid_rows(int n) { return n < 1 ? 1 : (n < kMaxGridY ? n : kMaxGridY); }
 template <typename R>
 cudaError_t launch_terrain(const float* dem, const float* terrain, int dem_pitch, int rows_full, int cols, int pitch,
                            int band_row0, int band_rows_pad, double cell, R* nx, R* ny, R* nz,

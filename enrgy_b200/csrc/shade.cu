@@ -10,7 +10,8 @@
 // cell (profiles/r01_summary.md: 750 instructions per cell-step on rough relief).
 //
 // Mapping: a THREAD owns V lines (l = Lw + 32 v + lane), their running maxima live in registers as
-// float64 (g is exact in float64, so the mask does not depend on rounding anywhere); a WARP owns the
+// float64 (u * dz is exact in float64 and g one correctly rounded subtraction, as in the oracle, so the
+// mask is the same on any hardware: DESIGN.md section 5); a WARP owns the
 // 32 V consecutive lines of its window and walks the rows from the sunward edge; the rows of the
 // terrain are read with coalesced (unaligned) 128-byte loads from a scan copy of the DEM with -inf
 // aprons (no bounds checks); the Q warps of a CTA sweep the same window for Q sub-steps of similar
@@ -55,20 +56,23 @@ __global__ void scan_fill_kernel(const float* __restrict__ src, int src_pitch, i
 __global__ void scan_transpose_kernel(const float* __restrict__ src, int src_pitch, int rows, int cols,
                                       float* __restrict__ scan_t, int pitch_t) {
   __shared__ float tile[32][33];
-  const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int r = r0 + i, c = c0 + threadIdx.x;
-    float v = -INFINITY;
-    if (r < rows && c < cols) {
-      const float z = src[(size_t)r * src_pitch + c];
-      if (z == z) v = z;
+  const int c0 = blockIdx.x * 32;
+  for (int r0 = blockIdx.y * 32; r0 < rows; r0 += gridDim.y * 32) {
+    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
+      const int r = r0 + i, c = c0 + threadIdx.x;
+      float v = -INFINITY;
+      if (r < rows && c < cols) {
+        const float z = src[(size_t)r * src_pitch + c];
+        if (z == z) v = z;
+      }
+      tile[i][threadIdx.x] = v;
     }
-    tile[i][threadIdx.x] = v;
-  }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int c = c0 + i, r = r0 + threadIdx.x;
-    if (c < cols && r < rows) scan_t[(size_t)(c + kScanRowApron) * pitch_t + kScanColApron + r] = tile[threadIdx.x][i];
+    __syncthreads();
+    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
+      const int c = c0 + i, r = r0 + threadIdx.x;
+      if (c < cols && r < rows) scan_t[(size_t)(c + kScanRowApron) * pitch_t + kScanColApron + r] = tile[threadIdx.x][i];
+    }
+    __syncthreads();                    // the tile is refilled by the next block of rows
   }
 }
 
@@ -125,11 +129,16 @@ __global__ void __launch_bounds__(32 * Q) sweep_kernel(const SweepArgs a) {
   // U rows per iteration; the loads of the NEXT iteration are issued before the current one is worked
   // on (two register buffers, the loop body exists twice), so a warp hides a full iteration of memory
   // latency by itself.  Rows past ua are inside the -inf aprons or harmless (nothing is emitted).
+  // The rows are loaded in the order u = ub, ub - 1, ub - 2, ...: their shears shear_q16(u, dfix) come from
+  // a running 64-bit accumulator q = u * dfix + 32768 (sh = q >> 16), one 64-bit subtraction per row
+  // instead of a 64-bit product (|u * dfix| reaches 2^36 on rasters of 2^20 cells a side).
+  long long q = (long long)ub * s.dfix + 32768;
   auto load_rows = [&](int u0, float (&h)[U][V], int (&col0)[U]) {
 #pragma unroll
     for (int i = 0; i < U; ++i) {
       const int u = u0 - i;
-      col0[i] = Lw + shear_q16(u, s.dfix);
+      col0[i] = Lw + (int)(q >> 16);
+      q -= s.dfix;
       const float* rowp = H + (long long)(s.sigma * u) * pitch + (col0[i] + lane);
 #pragma unroll
       for (int v = 0; v < V; ++v) h[i][v] = __ldg(rowp + 32 * v);
@@ -315,8 +324,8 @@ cudaError_t launch_scan_prepare(const float* src, int src_pitch, int rows, int c
   scan_fill_kernel<<<1184, 256, 0, stream>>>(src, src_pitch, rows, cols, scan, ps, ns);
   // the transposed copy: aprons by the same fill (no source), interior by the tile transpose
   scan_fill_kernel<<<1184, 256, 0, stream>>>(src, src_pitch, 0, 0, scan_t, pt, nt);
-  scan_transpose_kernel<<<dim3((cols + 31) / 32, (rows + 31) / 32), dim3(32, 8), 0, stream>>>(src, src_pitch, rows, cols,
-                                                                                             scan_t, pt);
+  scan_transpose_kernel<<<dim3((cols + 31) / 32, grid_rows((rows + 31) / 32)), dim3(32, 8), 0, stream>>>(
+      src, src_pitch, rows, cols, scan_t, pt);
   return cudaGetLastError();
 }
 
@@ -327,7 +336,10 @@ cudaError_t launch_sweep(const SweepArgs& a, int sm_count, cudaStream_t stream, 
   static_assert((long long)Q * 65535 >= kSweepMaxRowSubs, "grid.y of the sweep");
   int n = 0;
   // line groups: windows of 32 V lines every 32 (V - 1) lines over [-sh_max, nb - sh_min); the shear
-  // spans at most the length of the sweep axis (|dfix| <= 65536)
+  // spans at most the length of the sweep axis (|dfix| <= 65536).  grid.x is under 2^21 / 224 + 4 for
+  // rasters of up to 2^20 cells a side (the x limit is 2^31 - 1); grid.y counts sub-steps only
+  // (kSweepMaxRowSubs); the transpose's grid.y = tmp_words / 32 <= 2^20 / 1024 and its grid.z counts
+  // sub-steps (kSweepMaxColSubs).
   auto groups = [&](int na, int nb) { return (nb + na + 32 * V) / (32 * (V - 1)) + 2; };
   if (a.n_row_subs > 0) {
     dim3 grid(groups(a.rows, a.cols), (a.n_row_subs + Q - 1) / Q);

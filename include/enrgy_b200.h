@@ -158,6 +158,11 @@ const char* enrgy_last_error(void);
 int enrgy_device_count(void);
 
 /* life cycle: replaces Energy.__init__ state allocation (model.py:74-80) ---------------------- */
+/* rows and cols must lie in 1 .. 1048576 (2^20), else ENRGY_ERR_ARG.  The bound keeps every int cell
+ * coordinate and the Q16 shear of the shading sweep far from overflow, keeps the float32 cell
+ * coordinates of the station blend exact (< 2^24) and u * dz of the sweep exact in float64.  Device
+ * memory binds long before it: a raster that does not fit fails with ENRGY_ERR_CUDA when its buffers
+ * are allocated (enrgy_set_dem and the calls after it). */
 int enrgy_create(int device, int rows, int cols, int precision, enrgy_ctx** out);
 int enrgy_destroy(enrgy_ctx* ctx);
 
