@@ -19,7 +19,7 @@
 //   msm.py:193-203          melt partition                                -> balance()
 //   msm.py:31-107           sub-surface conduction (MSM variants)         -> balance()
 //   model.py:258-261        state update                                  -> balance(), epilogue
-//   var_classes.py:45-56, model.py:246-252  per-step area statistics      -> warp_reduce8 + slots + finalize
+//   var_classes.py:45-56, model.py:246-252  per-step area statistics      -> batch_put / batch_reduce + slots + finalize
 #include "kernels.cuh"
 
 #include <cstdio>
@@ -209,11 +209,99 @@ __device__ __forceinline__ float fmin_(float a, float b) { return fminf(a, b); }
 __device__ __forceinline__ double fmax_(double a, double b) { return fmax(a, b); }
 __device__ __forceinline__ double fmin_(double a, double b) { return fmin(a, b); }
 
+// ---- per-step area statistics: warp sums in batches of steps ------------------------------------
+// Every step a lane parks its NQ per-step values (one "entry"; with fused members one per (step, member)
+// pair) in its warp's batch buffer.  Once E entries are parked, lane r adds the 32 lane values of row
+// r = entry * NQ + statistic and writes that row's slot: per step NQ stores instead of a shuffle butterfly
+// (its shuffles, selects and chain of five shuffle latencies).  The sum adds lanes l and l ^ 16 first, then
+// ^ 8, ^ 4, ^ 2, ^ 1: the tree a butterfly over the lanes forms, so the sums are the same bits whichever
+// way they are formed, and deterministic.
+// Layout: [chunk][row][16 bytes], a chunk being the values of 16 / sizeof(R) consecutive lanes.  The row
+// pitch is odd (in chunks): a warp's stores of one row, and a quarter warp's 16-byte loads of one chunk of
+// eight consecutive rows, meet every bank at most once.
+__host__ __device__ constexpr int stat_batch_pitch(int rows) { return (rows | 1) * 16; }   // bytes between chunks
+__host__ __device__ constexpr int stat_batch_bytes(int r_size, int rows) {                  // per warp
+  return 32 / (16 / r_size) * stat_batch_pitch(rows);
+}
+template <typename R, int NQ, int E>
+struct StatBatch {
+  static constexpr int kRows = E * NQ;
+  static constexpr int kPitch = stat_batch_pitch(kRows);
+  static constexpr int kLanesPerChunk = 16 / (int)sizeof(R);
+  static constexpr int kBytes = stat_batch_bytes((int)sizeof(R), kRows);
+  static_assert(E >= 1 && kRows <= 32, "one row per lane");
+};
+// Statistic q of a batch entry is slot column stat_column(q): without the station blend the longwave
+// column (K_LWD) is not summed in the kernel (finalize_stats_kernel takes it from the DEM moments), so the
+// batch leaves it out.  Columns kStatsK + M_* are the sub-surface model's.
+template <bool LWD>
+__host__ __device__ constexpr int stat_column(int q) { return LWD || q < K_LWD ? q : q + 1; }
+// where lane `lane` parks its value of row 0
+template <typename R, int NQ, int E>
+__device__ __forceinline__ int batch_lane(int lane) {
+  using B = StatBatch<R, NQ, E>;
+  return lane / B::kLanesPerChunk * B::kPitch + lane % B::kLanesPerChunk * (int)sizeof(R);
+}
+template <typename R, int NQ>
+__device__ __forceinline__ void batch_put(unsigned char* lane_buf, int entry, const R (&v)[NQ]) {
+#pragma unroll
+  for (int q = 0; q < NQ; ++q) *reinterpret_cast<R*>(lane_buf + (entry * NQ + q) * 16) = v[q];
+}
+// the 32 lane values of the row whose chunk 0 is at `row`, added in the tree order above (packed adds:
+// pair i holds lanes 2i, 2i + 1)
+template <int PITCH>
+__device__ __forceinline__ float lane_sum(const unsigned char* row, float) {
+  V2<float> a[8];                                   // lanes (2i, 2i + 1) + (2i + 16, 2i + 17)
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    const ulonglong2 x = *reinterpret_cast<const ulonglong2*>(row + c * PITCH);
+    const ulonglong2 y = *reinterpret_cast<const ulonglong2*>(row + (c + 4) * PITCH);
+    a[2 * c] = add2(V2<float>{x.x}, V2<float>{y.x});
+    a[2 * c + 1] = add2(V2<float>{x.y}, V2<float>{y.y});
+  }
+#pragma unroll
+  for (int h = 4; h > 0; h >>= 1) {
+#pragma unroll
+    for (int i = 0; i < h; ++i) a[i] = add2(a[i], a[i + h]);
+  }
+  return a[0].lo() + a[0].hi();
+}
+template <int PITCH>
+__device__ __forceinline__ double lane_sum(const unsigned char* row, double) {
+  double a[16];                                     // lanes i + (i + 16)
+#pragma unroll
+  for (int c = 0; c < 8; ++c) {
+    const double2 x = *reinterpret_cast<const double2*>(row + c * PITCH);
+    const double2 y = *reinterpret_cast<const double2*>(row + (c + 8) * PITCH);
+    a[2 * c] = x.x + y.x;
+    a[2 * c + 1] = x.y + y.y;
+  }
+#pragma unroll
+  for (int h = 8; h > 0; h >>= 1) {
+#pragma unroll
+    for (int i = 0; i < h; ++i) a[i] += a[i + h];
+  }
+  return a[0];
+}
+// sums the first n_entries entries of the batch into their slots: statistic q of entry e goes to column
+// c = stat_column<LWD>(q), slots[e * kStatsK + c] (c < kStatsK) or slots_m[e * kStatsM + c - kStatsK].  The
+// caller orders it after the lanes' batch_put and before the next batch_put with __syncwarp.
+template <typename R, int NQ, int E, bool LWD>
+__device__ __forceinline__ void batch_reduce(const unsigned char* warp_buf, int n_entries, int lane, R* slots, R* slots_m) {
+  if (lane < n_entries * NQ) {
+    const int e = lane / NQ, c = stat_column<LWD>(lane - e * NQ);
+    const R v = lane_sum<StatBatch<R, NQ, E>::kPitch>(warp_buf + lane * 16, R{});
+    if (c < kStatsK) slots[e * kStatsK + c] = v;
+    else slots_m[e * kStatsM + (c - kStatsK)] = v;
+  }
+}
+
 // Sum of 8 per-thread values over the 32 lanes with 15 shuffles instead of 40: each butterfly stage
 // halves the number of values a lane still carries.  Returns the total of statistic
-// stat_of_lane(lane) = 4*bit4 + 2*bit3 + bit2; fixed order, hence deterministic.
+// stat_of_lane(lane) = 4*bit4 + 2*bit3 + bit2; the same tree as the batches', hence the same bits.  For the
+// kernel instances whose shared memory has no room for a batch buffer (StatBatchFor).
 template <typename R>
-__device__ __forceinline__ R warp_reduce8(const R (&v)[8], int lane) {
+__device__ __forceinline__ R warp_reduce8(const R* v, int lane) {   // v[0 .. 7]
   const unsigned full = 0xffffffffu;
   R a[4], b[2], c;
   bool hi = (lane & 16) != 0;
@@ -538,7 +626,7 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // run-time values chosen by the host (64 / 256, grown to the largest sub-step count of one step).
 template <typename R>
 struct SmemPlan {
-  int steps, subs, members, stations, slots, slots_m, ring, full, total;   // byte offsets and the total size
+  int steps, subs, members, stations, slots, slots_m, batch, ring, full, total;   // byte offsets and the total size
 };
 // nm: ensemble members fused into one pass (1 = a plain run: no member records); ns: weather stations
 // blended (1 = the reference's single AWS: no station records)
@@ -552,10 +640,11 @@ struct SmemPlan {
 template <typename R, bool MSM, int NM, int INSOL>
 constexpr bool kOneBarrier = ENRGY_ONE_BARRIER && sizeof(R) == 4 && !MSM && NM == 1 && INSOL == kInsolMasked;
 
+// batch_bytes: the warps' statistics batch buffers (StatBatchFor)
 template <typename R>
-__host__ __device__ inline SmemPlan<R> smem_plan(int warps, int cap_steps, int cap_subs, bool with_subs, bool msm,
-                                                 int nm = 1, int ns = 1, bool with_masks = false) {
-  SmemPlan<R> p;
+__host__ __device__ constexpr SmemPlan<R> smem_plan(int warps, int cap_steps, int cap_subs, bool with_subs, bool msm,
+                                                    int nm, int ns, bool with_masks, int batch_bytes) {
+  SmemPlan<R> p{};
   int o = 0;
   p.steps = o;   o += 2 * cap_steps * (int)sizeof(StepRec<R>);
   p.subs = o;    o += with_subs ? 2 * cap_subs * (int)sizeof(SubRec<R>) : 0;
@@ -565,6 +654,7 @@ __host__ __device__ inline SmemPlan<R> smem_plan(int warps, int cap_steps, int c
   p.slots = o;   o += (two_sets ? 2 : 1) * warps * cap_steps * nm * kStatsK * (int)sizeof(R);
   p.slots_m = o; o += msm ? warps * cap_steps * kStatsM * (int)sizeof(R) : 0;
   o = (o + 15) / 16 * 16;
+  p.batch = o;   o += batch_bytes;
   p.ring = o;    o += (ENRGY_MASK_RING && with_masks) ? warps * kRingSlots * 32 : 0;
   p.full = o;    o += 16;
   p.total = (o + 127) / 128 * 128;
@@ -603,6 +693,38 @@ constexpr int kMaskAhead = ENRGY_MASK_AHEAD;   // sunlit masks are prefetched th
 #ifndef ENRGY_MINB_MEMBERS
 #define ENRGY_MINB_MEMBERS 3
 #endif
+// Statistics batch of a kernel instance: entries per batch (0: no buffer, the warp reduces every step with
+// warp_reduce8) and the values of an entry.  The batch is as large as one row per lane allows (float64:
+// half the lanes), but never so large that the buffer costs the instance a CTA per SM at the default
+// time-block capacities: CTAs per SM by shared memory (228 KB per SM, 1 KB of it reserved per CTA) stay at
+// least what they were without the buffer, up to the launch bounds' minimum.  Where even one entry costs a
+// CTA (float64 with four fused members or with the station blend and its sub-step records), the instance
+// keeps the butterfly.
+template <typename R, int INSOL, bool MSM, bool DUMP, int NM, bool STATS, int NS>
+struct StatBatchFor {
+  static constexpr bool kLwd = NS > 1;                                   // K_LWD summed in the kernel
+  static constexpr int NQ = kStatsK - (kLwd ? 0 : 1) + (MSM ? kStatsM : 0);
+  static constexpr int W = kWarpsFor<R, INSOL>;
+  static constexpr int kMinCtas = NM > 2 ? ENRGY_MINB_MEMBERS : sizeof(R) == 4 ? ENRGY_MINB32 : ENRGY_MINB64;
+  static constexpr int bytes(int e) { return e > 0 ? W * stat_batch_bytes((int)sizeof(R), e * NQ) : 0; }
+  static constexpr int ctas(int e) {
+    return 233472 / (smem_plan<R>(W, kStepsPerBlock, kSubsPerBlock, INSOL != kInsolStreamed, MSM, NM, NS,
+                                  INSOL == kInsolMasked, bytes(e)).total + 1024);
+  }
+  static constexpr int pick() {
+    // (the sub-surface model: its batches added spills to three of its instances in ptxas)
+    if (!STATS || DUMP || MSM) return 0;
+    const int target = ctas(0) < kMinCtas ? ctas(0) : kMinCtas;
+    // (with sunlit masks at most 2 entries, summed at the end of the step: every arrangement with more spills
+    // in ptxas -- the mask loads keep more registers live through the step)
+    const int most = INSOL == kInsolMasked ? 2 : (sizeof(R) == 4 ? 32 : 16) / NQ;
+    for (int e = most; e > 0; --e)
+      if (ctas(e) >= target) return e;
+    return 0;
+  }
+  static constexpr int kEntries = pick();
+  static constexpr int kBytes = bytes(kEntries);                         // per CTA
+};
 // STATS = false (fused members only): no per-step area statistics -- their adds and the warp butterfly
 // are a third of a member's share of a step; the season totals come from the final rasters instead.
 // NS > 1: up to NS weather stations blended per cell (BASELINE config C4; specification in
@@ -623,7 +745,9 @@ energy_balance_kernel(const KernelArgs<R> a) {
   constexpr int NT = 32 * W;                       // threads per CTA
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int cap_steps = a.cap_steps, cap_subs = a.cap_subs;
-  const SmemPlan<R> plan = smem_plan<R>(W, cap_steps, cap_subs, INSOL != kInsolStreamed, MSM, NM, NS, INSOL == kInsolMasked);
+  using SB = StatBatchFor<R, INSOL, MSM, DUMP, NM, STATS, NS>;
+  const SmemPlan<R> plan = smem_plan<R>(W, cap_steps, cap_subs, INSOL != kInsolStreamed, MSM, NM, NS, INSOL == kInsolMasked,
+                                         SB::kBytes);
   StationRec<R>* const sm_stations = reinterpret_cast<StationRec<R>*>(smem_raw + plan.stations);  // [2][cap_steps][NS]
   StepRec<R>* const sm_steps = reinterpret_cast<StepRec<R>*>(smem_raw + plan.steps);     // [2][cap_steps]
   SubRec<R>* const sm_subs = reinterpret_cast<SubRec<R>*>(smem_raw + plan.subs);         // [2][cap_subs]
@@ -636,6 +760,11 @@ energy_balance_kernel(const KernelArgs<R> a) {
 
   constexpr int TILE_H = WY * KT, TILE_W = 32 * WX;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  // this warp's statistics batch: NQ values per entry, E entries (E = 0: no batch, warp_reduce8 per step)
+  constexpr int NQ = SB::NQ, E = SB::kEntries;
+  const int batch_off = plan.batch + warp * (SB::kBytes / W);               // byte offsets in smem_raw
+  int batch_mine = batch_off;                                                 // ... of this lane's value of row 0
+  if constexpr (E > 0) batch_mine += batch_lane<R, NQ, E>(lane);
   const R qnan = (R)__int_as_float(0x7fc00000);
 
   if (tid == 0) {
@@ -857,7 +986,18 @@ energy_balance_kernel(const KernelArgs<R> a) {
       // The step loop exists twice: for patches without off-glacier cells (no masking of the
       // statistics, so the whole balance of a step is one basic block the scheduler can interleave
       // freely: +3 %) and for patches with some.  (Reducing the statistics one step late, so that the
-      // shuffle butterfly of step t - 1 overlaps the balance of step t, measured 1 % slower.)
+      // shuffle butterfly of step t - 1 overlapped the balance of step t, measured 1 % slower.)
+      // Statistics batch: batch_n entries, the last of them entry `end - 1` of the block's slots, are parked in the warp's batch buffer.
+      int batch_n = 0;
+      auto flush_batch = [&](int end) {
+        const int e0 = end - batch_n;
+        __syncwarp();
+        if constexpr (E > 0)
+        batch_reduce<R, NQ, E, SB::kLwd>(smem_raw + batch_off, batch_n, lane, sm_slots + ((size_t)warp * cap_steps * NM + e0) * kStatsK,
+                            sm_slots_m + ((size_t)warp * cap_steps + e0) * kStatsM);
+        __syncwarp();                                  // read before the next entries overwrite them
+        batch_n = 0;
+      };
       auto run_steps = [&](auto full_tag) {
       constexpr bool FULL = decltype(full_tag)::value;
       // the codes that steer a step (sub-step range, albedo bracket and weight) are read one step
@@ -866,6 +1006,11 @@ energy_balance_kernel(const KernelArgs<R> a) {
       int sub_next = step_code(steps_b[ts].sub), pair_next = step_code(steps_b[ts].alb_pair);
       R w_next = steps_b[ts].alb_w;
       for (int t = ts; t < te; ++t) {
+        // a full batch is summed before the next step rather than at the end of the last one: there the
+        // next step's records and the step's own temporaries are live, and the 32 loaded values spill
+        if constexpr (E > 0 && NM <= E && INSOL != kInsolMasked) {
+          if (batch_n + NM > E) flush_batch((t - tb.t_begin) * NM);
+        }
         const StepRec<R> s = steps_b[t];
         const int sub_code = sub_next, pair = pair_next;
         const R alb_w = w_next;
@@ -1293,12 +1438,12 @@ energy_balance_kernel(const KernelArgs<R> a) {
           tic2[m][q] = add2(tic2[m][q], ice);
           }  // members
         }
-        // ---- per-step statistics: warp butterfly, one slot per warp (and member) -------------------
+        // ---- per-step statistics: one batch entry per member, summed over the warp per batch ----------
         if (!DUMP && STATS) {
           const R sum_sens = acc_sens.lo() + acc_sens.hi(), sum_lat = acc_lat.lo() + acc_lat.hi();
 #pragma unroll
           for (int m = 0; m < NM; ++m) {
-            R acc[kStatsK];
+            R acc[kStatsP];                            // by slot column
             acc[K_RS] = acc_rs[m].lo() + acc_rs[m].hi();
             acc[K_LWD] = NS > 1 ? acc_lwd.lo() + acc_lwd.hi() : (R)0;
             acc[K_SENS] = sum_sens;
@@ -1307,20 +1452,32 @@ energy_balance_kernel(const KernelArgs<R> a) {
             acc[K_SNOW] = acc_snow[m].lo() + acc_snow[m].hi();
             acc[K_SWE] = acc_swe[m].lo() + acc_swe[m].hi();
             acc[K_NSNOW] = (R)n_snow[m];
-            const R tot = warp_reduce8<R>(acc, lane);
-            if ((lane & 3) == 0)
-              sm_slots[((warp * cap_steps + (t - tb.t_begin)) * NM + m) * kStatsK + stat_of_lane(lane)] = tot;
-          }
-          if (MSM) {
-            R acc_m[kStatsM];
-            acc_m[M_LWU] = acc_lwu.lo() + acc_lwu.hi();
-            acc_m[M_G] = acc_g.lo() + acc_g.hi();
+            if constexpr (MSM) {
+              acc[kStatsK + M_LWU] = acc_lwu.lo() + acc_lwu.hi();
+              acc[kStatsK + M_G] = acc_g.lo() + acc_g.hi();
+            }
+            if constexpr (E > 0) {
+              R v[NQ];
 #pragma unroll
-            for (int q = 0; q < kStatsM; ++q) {
-              R v = acc_m[q];
+              for (int q = 0; q < NQ; ++q) v[q] = acc[stat_column<SB::kLwd>(q)];
+              batch_put<R, NQ>(smem_raw + batch_mine, batch_n, v);
+              ++batch_n;
+              if constexpr (NM > E || INSOL == kInsolMasked) {
+                if (batch_n == E) flush_batch((t - tb.t_begin) * NM + m + 1);
+              }
+            } else {
+              const R tot = warp_reduce8<R>(acc, lane);
+              if ((lane & 3) == 0)
+                sm_slots[((warp * cap_steps + (t - tb.t_begin)) * NM + m) * kStatsK + stat_of_lane(lane)] = tot;
+              if constexpr (MSM) {
 #pragma unroll
-              for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-              if (lane == 0) sm_slots_m[(warp * cap_steps + (t - tb.t_begin)) * kStatsM + q] = v;
+                for (int q = 0; q < kStatsM; ++q) {
+                  R x = acc[kStatsK + q];
+#pragma unroll
+                  for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+                  if (lane == 0) sm_slots_m[(warp * cap_steps + (t - tb.t_begin)) * kStatsM + q] = x;
+                }
+              }
             }
           }
         }
@@ -1432,6 +1589,7 @@ energy_balance_kernel(const KernelArgs<R> a) {
       }  // steps of the time block
       };
       if (patch_full) run_steps(std::true_type{}); else run_steps(std::false_type{});
+      if (!DUMP && STATS && E > 0 && batch_n > 0) flush_batch((te - tb.t_begin) * NM);   // the block's last, partial batch
 
       // ---- flush the block's statistics into this CTA's partial rows (fixed order) ---------------
       __syncthreads();
@@ -1442,6 +1600,7 @@ energy_balance_kernel(const KernelArgs<R> a) {
         for (int idx = tid; idx < n; idx += NT) {
           const int step = idx / NQ, q = idx - step * NQ;
           const int sl = (ts - tb.t_begin) * NM + step;
+          if (NS == 1 && q == K_LWD) continue;         // (no station blend: the column is not summed here)
           double sum = 0.0;
 #pragma unroll
           for (int w = 0; w < W; ++w) {
@@ -1524,7 +1683,8 @@ static cudaError_t configure(Instance<INSOL, MSM, DUMP, NM, STATS, NS>, int sm_c
                              LaunchInfo* info) {
   constexpr int K = PassShape<R, MSM, NM, NS>::K, KT = PassShape<R, MSM, NM, NS>::KT;
   auto kern = energy_balance_kernel<R, K, INSOL, MSM, DUMP, NM, KT, STATS, NS>;
-  const int smem = smem_plan<R>(kWarpsFor<R, INSOL>, cap_steps, cap_subs, INSOL != kInsolStreamed, MSM, NM, NS, INSOL == kInsolMasked).total;
+  const int smem = smem_plan<R>(kWarpsFor<R, INSOL>, cap_steps, cap_subs, INSOL != kInsolStreamed, MSM, NM, NS, INSOL == kInsolMasked,
+                                StatBatchFor<R, INSOL, MSM, DUMP, NM, STATS, NS>::kBytes).total;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;
   int per_sm = 0;
